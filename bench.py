@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Contract benchmark: GAT layer fwd+bwd edges/sec at the ogbn-proteins shape.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One "step" = one forward + backward of the GATConv sparse section (logits -> leaky_relu
 -> edge-softmax -> dropout -> SpMM -> scaling; SURVEY.md section 8d) over the whole
@@ -16,6 +16,10 @@ reduce-scattered back (bot_b200/partition.py).
 --impl reference: the oracle port of the reference math (pure torch, CPU) on a bounded
 sample of the same workload, on the host cores of this box (DGL itself is not
 installable offline: DESIGN.md).
+
+--dump-outputs DIR: after the timed steps, the results of the last one (the layer output and
+the gradients of its inputs) are written as DIR/<name>.npy; the inputs are seeded, so two
+builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -368,6 +372,8 @@ def run_ours(args):
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise RuntimeError("bench.py (impl ours) needs a CUDA device: bot_b200 has no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the results of one process: run it without torch.distributed")
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     host_affinity = pin_to_gpu_numa(local_rank, world)
@@ -459,8 +465,8 @@ def run_ours(args):
     sampler.mark_begin()
     barrier()
     e0.record()
-    for _ in range(args.steps):
-        step_resident()
+    for i in range(args.steps):
+        last = step_resident(keep_grads=bool(args.dump_outputs) and i == args.steps - 1)
     e1.record()
     barrier()
     sampler.mark_end()
@@ -474,6 +480,12 @@ def run_ours(args):
     ms_step = ms_total / args.steps
     total_edges = n_edges * (world if replicas else 1)
     value = total_edges / (ms_step * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"out": last[0], "grad_ft": ft_own.grad, "grad_el": el_own.grad,
+                                         "grad_er": None if er is None else er.grad}, {"grad_ee": None if ee is None else ee.grad})
+        del last
+        for t in leaves:
+            t.grad = None
 
     # per-kernel durations: a SECOND, instrumented pass of the same steps (CUDA events around every ABI call, the backward
     # issued as three calls) — outside the headline's timed region
@@ -622,6 +634,30 @@ def run_ours(args):
         emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, node_arrays, edge_arrays, max_rows=8192, max_edges=1 << 19, max_bytes=64 << 20):
+    """--dump-outputs: write every array that is not None as <out_dir>/<name>.npy in float32.  Node-indexed arrays
+    longer than ``max_rows`` keep the same seeded sample of rows, edge-indexed ones longer than ``max_edges`` the same
+    seeded sample of edges (canonical edge order), so that the files stay small (about 50 MB at every shape) and two
+    runs with the same arguments write the same rows."""
+    import numpy as np
+
+    out = {}
+    for arrays, cap in ((node_arrays, max_rows), (edge_arrays, max_edges)):
+        arrays = {k: v for k, v in arrays.items() if v is not None}
+        if not arrays:
+            continue
+        n = next(iter(arrays.values())).shape[0]
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:cap].sort().values if n > cap else None
+        for name, t in arrays.items():
+            out[name] = (t if idx is None else t[idx.to(t.device)]).detach().float().cpu().numpy()
+    total = sum(a.nbytes for a in out.values())
+    if total > max_bytes:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {max_bytes}-byte cap")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def parity_check(graph, src, dst, n_nodes, c, ft, el, er, ee, gout, cs, ds, step, dev, n_v=400, n_u=6):
@@ -864,7 +900,13 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="developer runs: skip the end-to-end leg")
     ap.add_argument("--no-e2e-model", action="store_true", help="skip the whole-model end-to-end line (proteins shape, 1 GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's layer output and input gradients (seeded sample) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

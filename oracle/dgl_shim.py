@@ -6,8 +6,8 @@ reference's ``models.py`` files cannot be imported as they are.  ``install()``
 registers a fake ``dgl`` package in ``sys.modules`` whose graph object implements —
 in plain differentiable torch ops on CPU — exactly the calls the reference's
 ``GATConv``/``GAT`` make (SURVEY.md section 2b K1-K13, Appendix B).  With it,
-``tests/golden/make_golden.py`` imports the UNMODIFIED reference modules from
-/root/reference and records their outputs, so the reference's own orchestration
+``tests/golden/make_golden.py`` imports the UNMODIFIED reference modules from a
+reference checkout and records their outputs, so the reference's own orchestration
 (aliasing before scaling, +0.5 exponent, in-place adds, randperm edge-drop ...)
 is what the golden vectors pin; only the DGL primitives are restated here.
 """
@@ -203,11 +203,15 @@ def install():
 
 def import_reference(which):
     """Import an unmodified reference ``models.py`` ('no-sampling', 'ogbn-proteins',
-    'ogbn-products') from /root/reference under a unique module name."""
+    'ogbn-products') of the reference checkout named by ``BOT_REFERENCE`` under a unique module name."""
     import importlib.util
+    import os
 
+    root = os.environ.get("BOT_REFERENCE")
+    if not root:
+        raise RuntimeError("set BOT_REFERENCE to a checkout of the reference (AiRyunn/BoT)")
     install()
-    path = f"/root/reference/src/{which}/models.py"
+    path = os.path.join(root, "src", which, "models.py")
     spec = importlib.util.spec_from_file_location(f"_bot_ref_{which.replace('-', '_')}", path)
     m = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(m)

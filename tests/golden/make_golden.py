@@ -1,8 +1,8 @@
 """Generate the golden vectors under tests/golden/ by running the UNMODIFIED reference modules
-(/root/reference/src/*/models.py) on CPU on top of oracle/dgl_shim.py (DGL itself is not installable
+(src/*/models.py of a reference checkout) on CPU on top of oracle/dgl_shim.py (DGL itself is not installable
 offline; the shim restates only the DGL primitives, SURVEY.md Appendix B).
 
-    python tests/golden/make_golden.py        # run in the build container; /root/reference is NOT on the GPU box
+    BOT_REFERENCE=<reference checkout> python tests/golden/make_golden.py
 
 Each case stores: the COO graph, the module's state_dict, the inputs, the output, the gradients of a fixed
 scalar loss w.r.t. the inputs and parameters, and — for training-mode cases — the random edge-drop permutation
