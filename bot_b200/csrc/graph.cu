@@ -49,7 +49,10 @@ Tiling choose_tiling(int H, int D, int64_t ld_g, const void* pg, int64_t ld_o, c
   if ((force_vw == 1 || force_vw == 2) && force_vw < t.vw) t.vw = force_vw;
   const int gline = 32 / t.vw;  // lanes that cover one 128-byte line
   // line-alignment shift is possible when every gathered row starts on a line boundary
-  const bool can_align = (ld_g * 4) % 128 == 0 && ((uintptr_t)pg % 128) == 0 && env_int("BOTGAT_NOALIGN", 0) == 0;
+  bool can_align = (ld_g * 4) % 128 == 0 && ((uintptr_t)pg % 128) == 0 && env_int("BOTGAT_NOALIGN", 0) == 0;
+  // a caller that needs the head in one part (the backward src pass) gives up the shift before the shift's extra
+  // line would push the head past one pass: 32 * kVplCap vectors instead of one line fewer
+  if (col_parts_req == 1 && can_align && D > (32 * kVplCap - gline) * t.vw) can_align = false;
   const int cap_cols = (32 * kVplCap - (can_align ? gline : 0)) * t.vw;  // widest part one warp covers in a pass
   int parts = col_parts_req;
   if (parts <= 0) {

@@ -324,6 +324,11 @@ def _backward_core(graph, cfg, pre, hooks, ft2d, el, er, ee, keep, attn_mul, src
     return grad_el, grad_er, (grad_ee if need_ee else None)
 
 
+# Widest head the backward src pass covers: one warp row of 32 lanes x 8 float4 vectors (csrc/graph.cu choose_tiling).
+# GATFusedFn zero-pads a head too wide for its vector width to a multiple of 4 columns, which gets float4 vectors.
+BWD_MAX_D = 1024
+
+
 class GATFusedFn(torch.autograd.Function):
     """out = dst_scale * sum_k softmax_v(leaky_relu(el[u]+er[v]+ee[k]))*attn_mul[k] * src_scale[u] * ft[u].
 
@@ -354,16 +359,30 @@ class GATFusedFn(torch.autograd.Function):
         er = None if er is None else _f32c(er, "er").view(N_d, H)
         ee, ld_ee, keep, attn_mul, ld_am = _check_edge_operands(graph, H, ee, keep, attn_mul)
         src_scale, dst_scale = _f32c(src_scale, "src_scale"), _f32c(dst_scale, "dst_scale")
+        Dk = D
+        if any(ctx.needs_input_grad):
+            if D > BWD_MAX_D:
+                raise ValueError(f"GAT layer with gradients: head width D={D} exceeds the backward's limit of {BWD_MAX_D} "
+                                 "columns per head (inference without gradients has no such limit)")
+            vw = 4 if D % 4 == 0 and ft.data_ptr() % 16 == 0 else 2 if D % 2 == 0 and ft.data_ptr() % 8 == 0 else 1
+            if D > 256 * vw:
+                # the src pass covers a head in one pass of 256 vectors of vw floats; a wider head is zero-padded to a
+                # multiple of 4 columns and gets float4 vectors (the padding adds zeros to every sum)
+                if hooks is not None:
+                    raise ValueError(f"GAT layer with hooks: D={D} > {256 * vw} needs a multiple of 4 and a 16-byte aligned ft")
+                Dk = _r4(D)
+                ft = torch.cat([ft, ft.new_zeros(N_s, H, Dk - D)], 2)
         with torch.cuda.device(ft.device):
             out, row_max, row_sum, pre, attn_p_used = _forward_core(
-                graph, ft.view(N_s, H * D), H, D, el, er, ee, ld_ee, keep, attn_mul, ld_am, src_scale, dst_scale, slope,
+                graph, ft.view(N_s, H * Dk), H, Dk, el, er, ee, ld_ee, keep, attn_mul, ld_am, src_scale, dst_scale, slope,
                 attn_p, seed, hooks, any(ctx.needs_input_grad))
         ctx.graph = graph
         ctx.hooks = hooks
         ctx.pre = pre
-        ctx.cfg = (H, D, edge_mode == "staged", float(slope), attn_p_used, int(seed))
+        ctx.D = D
+        ctx.cfg = (H, Dk, edge_mode == "staged", float(slope), attn_p_used, int(seed))
         ctx.save_for_backward(ft, el, er, ee, keep, attn_mul, src_scale, dst_scale, out, row_max, row_sum)
-        return out
+        return out if Dk == D else out[:, :, :D].contiguous()
 
     @staticmethod
     def backward(ctx, gout):
@@ -372,11 +391,17 @@ class GATFusedFn(torch.autograd.Function):
         need_er = er is not None and ctx.needs_input_grad[3]
         need_ee = ee is not None and ctx.needs_input_grad[4]
         gout = _f32c(gout, "grad_out")
+        if D != ctx.D:     # zero-padded head (see forward)
+            gout = torch.cat([gout, gout.new_zeros(gout.shape[0], H, D - ctx.D)], 2)
+        elif D > 256 and gout.data_ptr() % 16:
+            gout = gout.clone()   # a 16-byte aligned g' keeps float4 vectors (one pass per head)
         grad_ft = torch.empty_like(ft)
         with torch.cuda.device(ft.device):
             grad_el, grad_er, grad_ee = _backward_core(
                 ctx.graph, ctx.cfg, ctx.pre, ctx.hooks, ft.view(-1, H * D), el, er, ee, keep, attn_mul, src_scale, dst_scale,
                 out, row_max, row_sum, gout, grad_ft.view(-1, H * D), need_er, need_ee, hook_grad_ft=grad_ft)
+        if D != ctx.D:
+            grad_ft = grad_ft[:, :, :ctx.D]
         return (None, grad_ft, grad_el, grad_er, grad_ee, None, None, None, None, None, None, None, None)
 
 
@@ -419,6 +444,10 @@ class GATConvSampledFn(torch.autograd.Function):
         bd = torch.cat([b_dst, b_dst.new_zeros(P - HD)])
         ee, ld_ee, keep, attn_mul, ld_am = _check_edge_operands(graph, H, ee, keep, attn_mul)
         dst_scale, src_scale = _f32c(dst_scale, "dst_scale"), _f32c(src_scale, "src_scale")
+        vw = 4 if D % 4 == 0 else 2 if D % 2 == 0 else 1
+        if any(ctx.needs_input_grad) and D > min(256 * vw, BWD_MAX_D):
+            raise ValueError(f"GAT layer with gradients: head width D={D} exceeds the backward's limit of {256 * vw} columns "
+                             f"per head at {vw}-float vectors (at most {BWD_MAX_D}, for D a multiple of 4)")
         with torch.cuda.device(x_src.device):
             Ys = x_src @ ws.t()
             Yd = torch.addmm(bd, x_dst, wd.t())

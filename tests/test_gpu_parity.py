@@ -121,15 +121,54 @@ def test_column_parts_forward(cuda, monkeypatch):
     assert rel_err(out, ref) <= FWD_TOL
 
 
+def _gather_kernels(fn):
+    """Normalised names of the gather kernels ``fn()`` launches (torch.profiler, CUDA activity)."""
+    from torch.profiler import ProfilerActivity, profile
+
+    from test_gpu_kernel_coverage import normalise
+
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    return {n for n in (normalise(e.name) for e in prof.events()) if n}
+
+
 def test_forced_group_sizes(cuda, monkeypatch):
-    c = make_case(300, 300, 20000, 2, 64, ee=True, seed=6)
-    ref, refg = oracle_run(c)
-    for G in (1, 2, 4, 8, 16, 32):
+    """BOTGAT_G forces the lanes per neighbour of the head-major kernels; each shape is one the forced G covers (one
+    vector slot per lane at G = D/4 and below), and the trace shows that G ran in both passes."""
+    monkeypatch.setenv("BOTGAT_LOWDEG", "0")
+    monkeypatch.setenv("BOTGAT_ROWWISE", "0")
+    monkeypatch.setenv("BOTGAT_BWD_TMA", "0")
+    for G, H, D in ((1, 2, 4), (2, 2, 8), (4, 2, 12), (8, 2, 16), (16, 2, 64), (32, 2, 64)):
+        c = make_case(300, 300, 20000, H, D, ee=True, seed=6)
         monkeypatch.setenv("BOTGAT_G", str(G))
-        out, g, _ = engine_run(c, cuda)
-        assert rel_err(out, ref) <= FWD_TOL, G
-        assert rel_err(g["ft"], refg["ft"]) <= 1e-4 and rel_err(g["el"], refg["el"]) <= 1e-4, G
-        assert rel_err(g["er"], refg["er"]) <= 1e-4 and rel_err(g["ee"], refg["ee"]) <= 1e-4, G
+        names = _gather_kernels(lambda: check_case(c, cuda))
+        gsh = G.bit_length() - 1
+        assert {n.split("<")[0] for n in names} == {"botgat::gat_fwd_kernel", "botgat::gat_bwd_src_kernel"}, (G, names)
+        assert all(n.split("<")[1].split(",")[1] == str(gsh) for n in names), (G, names)
+
+
+@pytest.mark.parametrize("D", [301, 514])
+def test_wide_heads_train(cuda, D):
+    """Heads wider than the backward covers at their vector width (odd D > 256, D = 2 mod 4 > 512) are zero-padded to a
+    multiple of 4 and train; the output and gradients keep the caller's width."""
+    c = make_case(150, 150, 2000, 1, D, ee=True, keep_p=0.1, seed=D)
+    check_case(c, cuda)
+
+
+def test_too_wide_heads_are_rejected(cuda):
+    """D > 1024 with gradients is rejected before any launch, naming the limit; with no input requiring grad it runs."""
+    import bot_b200
+    from bot_b200.functional import gat_fused
+
+    c = make_case(50, 50, 300, 1, 1100, seed=3)
+    g = bot_b200.Graph(c["src"].to(cuda), c["dst"].to(cuda), 50)
+    ft = c["ft"].to(cuda).requires_grad_(True)
+    with pytest.raises(ValueError, match="1024"):
+        gat_fused(g, ft, c["el"].to(cuda), c["er"].to(cuda))
+    out = gat_fused(g, ft.detach(), c["el"].to(cuda), c["er"].to(cuda))
+    ref, _ = oracle_run(c)
+    assert rel_err(out, ref) <= FWD_TOL
 
 
 def test_deterministic(cuda):
@@ -805,7 +844,7 @@ def test_v1_folded_logits_match_unfolded(cuda, kind):
         assert rel_err(gp1[k], gp2[k]) <= 1e-4, k
 
 
-@pytest.mark.parametrize("tma", ["0", "1", "2"])
+@pytest.mark.parametrize("tma", ["0", "1"])
 @pytest.mark.parametrize("H,D,kw", [
     (6, 80, dict(ee=True, keep_p=0.1)),              # proteins: G = 4, five slots, no idle lanes
     (4, 64, dict(er=False, symm=True, attn_p=0.1)),  # Reddit
@@ -813,10 +852,14 @@ def test_v1_folded_logits_match_unfolded(cuda, kind):
     (2, 16, dict()), (3, 32, dict(ee=True)), (2, 48, dict()), (1, 96, dict(symm=True)), (2, 128, dict(ee=True)),
     (3, 40, dict(er=False)), (1, 160, dict(ee=True, keep_p=0.3)),
     (2, 72, dict(ee=True)),                          # a width the TMA kernel is not instantiated for: LDG either way
+    (12, 32, dict(ee=True)), (12, 120, dict(keep_p=0.2)),   # H > 8: edge records wider than one 32-byte sector
+    (5, 40, dict(ee=True, keep_p=0.1)), (8, 16, dict(er=False, attn_p=0.2)), (1, 128, dict(er=False, symm=True)),
+    (3, 160, dict(attn_p=0.1)),
 ])
 def test_src_pass_tma_and_ldg(cuda, monkeypatch, tma, H, D, kw):
-    """The warp-per-row backward src pass in both data-movement variants (TMA gather4 ring / LDG registers) on every
-    head width the TMA kernels (1 = a block per row, 2 = persistent warps) are instantiated for: rows of 0, 1, < 32, exactly 32/64 and several hundred out-edges."""
+    """The warp-per-row backward src pass in both data-movement variants (BOTGAT_BWD_TMA unset or 1: the TMA gather4
+    ring; 0: LDG into registers) on every head width the TMA kernel is instantiated for, and D = 72, which it is not (LDG
+    either way): rows of 0, 1, < 32, exactly 32/64 and several hundred out-edges.  The trace shows which one ran."""
     monkeypatch.setenv("BOTGAT_LOWDEG", "0")
     monkeypatch.setenv("BOTGAT_BWD_TMA", tma)
     n = 260
@@ -830,7 +873,10 @@ def test_src_pass_tma_and_ldg(cuda, monkeypatch, tma, H, D, kw):
     if c["src_scale"] is not None:
         f = graph_ref.build_formats(c["src"].numpy(), c["dst"].numpy(), n, n)
         c["src_scale"] = torch.from_numpy(graph_ref.deg_scale(f["out_deg"], -0.5))
-    check_case(c, cuda)
+    names = _gather_kernels(lambda: check_case(c, cuda))
+    src = {n.split("<")[0] for n in names if "bwd" in n}
+    want = "botgat::gat_bwd_src_tma_kernel" if tma == "1" and D != 72 else "botgat::gat_bwd_src_kernel"
+    assert src == {want}, (tma, D, names)
 
 
 @pytest.mark.parametrize("tma", ["1", "2"])
@@ -943,12 +989,18 @@ ROWWISE_CASES.update({
 def test_rowwise_kernels(cuda, monkeypatch, name, bulk):
     """One warp per row for all heads (forward and backward src pass; the latter with its rows staged by bulk copies
     into a shared-memory ring, or through the register ring) against the fp64 oracle on every parity case; shapes the
-    family does not cover (vector width < 4) silently take the head-major kernels."""
+    family does not cover (vector width < 4) take the head-major kernels.  The trace shows which family ran."""
     monkeypatch.setenv("BOTGAT_ROWWISE", "1")
     monkeypatch.setenv("BOTGAT_RW_BULK", bulk)
     n_src, n_dst, e, H, D, kw = ROWWISE_CASES[name]
     c = make_case(n_src, n_dst, e, H, D, seed=zlib.crc32(name.encode()) % 1000 + 2, **kw)
-    check_case(c, cuda)
+    names = _gather_kernels(lambda: check_case(c, cuda))
+    families = {n.split("<")[0] for n in names}
+    if D % 4 == 0 and H <= 8 and D // 4 <= 8 * (32 // (1 << (H - 1).bit_length())):
+        assert families == {"botgat::gat_fwd_rowwise_kernel",
+                            "botgat::gat_bwd_src_rowbulk_kernel" if bulk == "1" else "botgat::gat_bwd_src_rowwise_kernel"}, names
+    else:
+        assert not any("rowwise" in f or "rowbulk" in f for f in families), names
     o1, g1, _ = engine_run(c, cuda)
     o2, g2, _ = engine_run(c, cuda)
     assert torch.equal(o1, o2) and all(g1[k] is None or torch.equal(g1[k], g2[k]) for k in g1)

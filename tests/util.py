@@ -100,16 +100,24 @@ def engine_run(c, device, slope=0.2, attn_p=0.0, seed=0):
 
 
 def check_case(c, device, **kw):
+    """Forward and gradients against the fp64 oracle, norm-relative and row-normalised (``gat_rows.row_rel_err``, each
+    row by its own magnitude floored at 1e-3 (forward) / 1e-2 (gradients) of the global one, as test_gpu_fullsize)."""
+    from oracle.gat_rows import row_rel_err
+
     ref_out, ref_g = oracle_run(c)
     out, g, _ = engine_run(c, device, **kw)
     errs = {"out": rel_err(out, ref_out)}
     assert errs["out"] <= FWD_TOL, f"forward rel err {errs['out']:.3e} > {FWD_TOL}"
+    r = row_rel_err(out, ref_out, 1e-3)
+    assert r <= FWD_TOL, f"forward row-normalised err {r:.3e} > {FWD_TOL}"
     for k in ("ft", "el", "er", "ee"):
         if ref_g[k] is None:
             assert g[k] is None
             continue
         errs[k] = rel_err(g[k], ref_g[k])
         assert errs[k] <= GRAD_TOL, f"grad_{k} rel err {errs[k]:.3e} > {GRAD_TOL}"
+        r = row_rel_err(g[k], ref_g[k], 1e-2)
+        assert r <= GRAD_TOL, f"grad_{k} row-normalised err {r:.3e} > {GRAD_TOL}"
     return errs
 
 
