@@ -6,11 +6,16 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <type_traits>
+
 #include "botgat.h"
 
 namespace botgat {
 
 void set_error(const char* fmt, ...);
+// host (plan.cu): environment variables; an unset or empty one reads as null / `dflt`
+const char* env_str(const char* name);
+int64_t env_int(const char* name, int64_t dflt);
 extern std::atomic<long long> g_launches;  // kernels launched by this library (botgat_launch_count)
 #define BG_LAUNCHED(n) (::botgat::g_launches.fetch_add(n, std::memory_order_relaxed))
 
@@ -231,11 +236,6 @@ struct Tiling {
   int omask;      // lane-offset mask: o = (first vector index of the slab) & omask; 0 = no alignment shift
 };
 
-// host: choose the tiling.  `ld_g`/`pg` describe the GATHERED table (alignment shift is derived from it),
-// `ld_o`/`po` the row-local one (only constrains the vector width).
-Tiling choose_tiling(int H, int D, int64_t ld_g, const void* pg, int64_t ld_o, const void* po, int col_parts_req,
-                     int64_t n_rows_table);
-
 // host (segments.cu): build / free the segment table of one CSR; a no-op when no row exceeds the segment length
 int build_segments(int n_rows, const int32_t* indptr, const int32_t* deg, int64_t max_deg, botgat_graph::SegTable* t,
                    cudaStream_t st);
@@ -279,8 +279,13 @@ __host__ __device__ constexpr int bwd_min_blocks(int vpl) { return vpl <= 3 ? BG
   BG_VPL_SMALL(X, 1, 0) BG_VPL_SMALL(X, 1, 1) BG_VPL_SMALL(X, 1, 2) BG_VPL_SMALL(X, 1, 3) BG_VPL_SMALL(X, 1, 4) \
   BG_VPL_FULL(X, 1, 5)
 
-inline bool combo_supported(int vw, int gsh, int vpl) {
-#define BG_X(VW, GSH, VPL) if (vw == VW && gsh == GSH && vpl == VPL) return true;
+// Calls f(VW, GSH, VPL), each a std::integral_constant, for the instantiated combination equal to (vw, gsh, vpl);
+// false when there is none.
+template <class F>
+inline bool with_combo(int vw, int gsh, int vpl, F&& f) {
+#define BG_X(VW, GSH, VPL)                                                                                          \
+  if (vw == VW && gsh == GSH && vpl == VPL)                                                                         \
+    return f(std::integral_constant<int, VW>(), std::integral_constant<int, GSH>(), std::integral_constant<int, VPL>()), true;
   BG_COMBOS(BG_X)
 #undef BG_X
   return false;

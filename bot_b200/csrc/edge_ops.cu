@@ -12,8 +12,7 @@
 namespace botgat {
 
 static int env_pf() {
-  const char* s = getenv("BOTGAT_PF");
-  return (s && *s) ? atoi(s) : 0;  // L2 prefetch-size hints measured neutral on B200 (profiles/r01_sweeps.md)
+  return (int)env_int("BOTGAT_PF", 0);  // L2 prefetch-size hints measured neutral on B200 (profiles/r01_sweeps.md)
 }
 
 template <int PF> __device__ __forceinline__ float4 ld_rec4(const float* p) {

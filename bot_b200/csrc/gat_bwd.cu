@@ -287,18 +287,14 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32, bwd_min_blocks(VPL)) gat_
   if (lane == 0) p.grad_el[(int64_t)row * p.H + h] = gel;
 }
 
-static int launch_src(const BwdParams& p, const Tiling& t, dim3 grid, cudaStream_t st) {
-  dim3 block(kWarpsPerBlock * 32);
-#define BG_X(VW, GSH, VPL)                                            \
-  if (t.vw == VW && t.gshift == GSH && t.vpl == VPL) {                \
-    gat_bwd_src_kernel<VW, GSH, VPL><<<grid, block, 0, st>>>(p);      \
-    BG_LAUNCHED(1);                                                   \
-    return 0;                                                         \
-  }
-  BG_COMBOS(BG_X)
-#undef BG_X
-  set_error("backward: no kernel for vw=%d lanes=%d slots=%d", t.vw, 1 << t.gshift, t.vpl);
-  return -1;
+static int launch_src(const BwdParams& p, const SrcPlan& plan, cudaStream_t st) {
+  const Tiling& t = plan.t;
+  const bool launched = with_combo(t.vw, t.gshift, t.vpl, [&](auto vw, auto gsh, auto vpl) {
+    gat_bwd_src_kernel<vw.value, gsh.value, vpl.value><<<plan.grid, kWarpsPerBlock * 32, 0, st>>>(p);
+  });
+  BG_REQUIRE(launched, "backward: no kernel for vw=%d lanes=%d slots=%d", t.vw, 1 << t.gshift, t.vpl);
+  BG_LAUNCHED(1);
+  return 0;
 }
 
 }  // namespace botgat
@@ -341,41 +337,25 @@ extern "C" int botgat_gat_backward(const botgat_graph* g, const botgat_bwd_args*
   const int64_t ld_gee = a->ld_gee > 0 ? a->ld_gee : a->H;
   BG_REQUIRE(a->gz || ld_gee == a->H, "backward: a padded grad_ee needs the staged path (gz workspace)");
 
-  const bool node_major = drec_node_major(a->H, a->D, g->n_dst, g->n_edges, g->n_src);
   BG_REQUIRE(g->n_dst * (int64_t)a->H < (1ll << 31), "backward: n_dst * H must be < 2^31");
-  const int drec_hs = node_major ? 1 : (int)g->n_dst, drec_vs = node_major ? a->H : 1;
-  if (phases & 1) {
-    dim3 grid((unsigned)((g->n_dst + kWarpsPerBlock - 1) / kWarpsPerBlock));
-    gat_bwd_node_kernel<<<grid, block, 0, st>>>((int)g->n_dst, a->H, a->D, a->ld_out, a->out, a->gout, a->er,
-                                                a->row_max, a->row_sum, a->dst_scale, (float4*)a->drec, drec_hs, drec_vs,
-                                                a->dst_scale ? a->gprime : nullptr);
-    BG_LAUNCHED(1);
-    BG_CHECK(cudaGetLastError());
-  }
   const float* gp = a->dst_scale ? a->gprime : a->gout;
-
-  if (phases & 2) {
-    BwdParams p;
+  BwdParams p;
+  SrcPlan plan;
+  if (phases & 3) {
+    // the src pass's plan also fixes the layout the node phase writes the records in
     p.n_dst = (int)g->n_dst; p.n_edges = g->n_edges;
     p.H = a->H; p.D = a->D; p.ld_ft = a->ld_ft; p.ld_g = a->ld_out; p.ld_gft = a->ld_gft;
     p.ft = a->ft; p.el = a->el; p.cs = a->src_scale; p.g = gp; p.drec = (const float4*)a->drec;
-    p.drec_hs = drec_hs; p.drec_vs = drec_vs;
     p.Hb = a->Hb; p.slope = a->slope; p.attn_p = a->attn_p; p.inv_keep = 1.f / (1.f - a->attn_p); p.seed = a->seed;
     p.grad_ft = a->grad_ft; p.grad_el = a->grad_el;
     p.ee = a->ee; p.keep = a->keep; p.amul_e = a->attn_mul;
     // grad_ee is written straight in edge-id order by the src pass unless the caller supplies the staged
     // workspace gz (then phase 4 un-stages it)
     p.gz = a->gz; p.gz_e = a->gz ? nullptr : a->grad_ee;
-    // the gathered table is g' (ld_out); ft and grad_ft are row-local and only constrain the vector width
-    const int64_t ld_o = a->ld_ft | a->ld_gft;  // low bits clear iff both are multiples of the vector width
-    const uintptr_t po = (uintptr_t)a->ft | (uintptr_t)a->grad_ft;
-    Tiling t = choose_tiling(a->H, a->D, a->ld_out, gp, ld_o, (const void*)po, 1, g->n_dst);
-    BG_REQUIRE(t.col_parts == 1, "backward: D=%d too wide for one pass (max %d)", a->D, 32 * 8 * t.vw);
     p.indptr = g->out_indptr; p.indices = g->out_indices; p.eid = g->out_eid;
-    p.n_rows = (int)g->n_src; p.eb = a->eb_out; p.am = a->am_out; p.omask = t.omask;
+    p.n_rows = (int)g->n_src; p.eb = a->eb_out; p.am = a->am_out;
     const botgat_graph::SegTable& seg = g->seg_out;
-    const bool lowdeg = use_lowdeg_kernels(g->n_edges, g->n_src, true);
-    const bool split = seg.n_items > 0;   // both kernel families work on (row | segment) items
+    const bool split = seg.n_items > 0;   // every kernel family works on (row | segment) items
     BG_REQUIRE(!split || seg.n_slots == 0 || a->scratch, "backward: this graph has split rows; scratch is required");
     p.seg_row = split ? seg.row : nullptr; p.seg_beg = seg.beg; p.seg_end = seg.end; p.seg_slot = seg.slot;
     p.n_items = split ? seg.n_items : p.n_rows; p.scratch = a->scratch;
@@ -384,25 +364,29 @@ extern "C" int botgat_gat_backward(const botgat_graph* g, const botgat_bwd_args*
     p.h_count = a->h_count > 0 ? a->h_count : a->H - a->h_begin;
     BG_REQUIRE(p.h_begin >= 0 && p.h_count > 0 && p.h_begin + p.h_count <= a->H, "backward: bad head range [%d, +%d) of %d", a->h_begin, a->h_count, a->H);
     BG_REQUIRE(!split || p.h_count == a->H, "backward: a graph with split rows needs the full head range");
-    const int64_t nblocks = (int64_t)p.blocks_per_slab * p.h_count;
-    BG_REQUIRE(nblocks < (1ll << 31), "backward: grid too large");
-    int rc = launch_src_rowwise(p, t, st);        // 1 = not wanted for this table size / shape not covered
-    if (rc == 1 && node_major) {
-      // The node phase laid the records out for the all-heads-per-row kernel, which does not cover this call after all
-      // (operands by edge id, an unaligned table): redo the cheap node phase head-major.  gprime is rewritten with
-      // the same values.
-      dim3 ngrid((unsigned)((g->n_dst + kWarpsPerBlock - 1) / kWarpsPerBlock));
-      gat_bwd_node_kernel<<<ngrid, block, 0, st>>>((int)g->n_dst, a->H, a->D, a->ld_out, a->out, a->gout, a->er, a->row_max,
-                                                   a->row_sum, a->dst_scale, (float4*)a->drec, (int)g->n_dst, 1,
-                                                   a->dst_scale ? a->gprime : nullptr);
-      BG_LAUNCHED(1);
-      BG_CHECK(cudaGetLastError());
-    }
-    if (rc == 1 && !lowdeg) rc = launch_src_tma(p, t, st);   // 1 = shape not covered by the TMA kernel
-    if (rc == 1) rc = lowdeg ? launch_src_lowdeg(p, t, st) : launch_src(p, t, dim3((unsigned)nblocks), st);
+    const int rc = plan_src(Knobs::read(), p, &plan);
     if (rc) return rc;
-    if (split) {
-      rc = launch_bwd_combine(seg, a->H, a->D, a->ld_gft, a->scratch, a->src_scale, a->grad_ft, a->grad_el, st);
+    p.omask = plan.t.omask;
+    p.drec_hs = plan.records_node_major ? 1 : (int)g->n_dst;
+    p.drec_vs = plan.records_node_major ? a->H : 1;
+  }
+  if (phases & 1) {
+    dim3 grid((unsigned)((g->n_dst + kWarpsPerBlock - 1) / kWarpsPerBlock));
+    gat_bwd_node_kernel<<<grid, block, 0, st>>>((int)g->n_dst, a->H, a->D, a->ld_out, a->out, a->gout, a->er,
+                                                a->row_max, a->row_sum, a->dst_scale, (float4*)a->drec, p.drec_hs, p.drec_vs,
+                                                a->dst_scale ? a->gprime : nullptr);
+    BG_LAUNCHED(1);
+    BG_CHECK(cudaGetLastError());
+  }
+
+  if (phases & 2) {
+    int rc = plan.family == Family::rowwise || plan.family == Family::rowbulk ? launch_src_rowwise(p, plan, st)
+             : plan.family == Family::tma                                     ? launch_src_tma(p, plan, st)
+             : plan.family == Family::lowdeg                                  ? launch_src_lowdeg(p, plan, st)
+                                                                              : launch_src(p, plan, st);
+    if (rc) return rc;
+    if (p.seg_row) {
+      rc = launch_bwd_combine(g->seg_out, a->H, a->D, a->ld_gft, a->scratch, a->src_scale, a->grad_ft, a->grad_el, st);
       if (rc) return rc;
     }
     BG_CHECK(cudaGetLastError());

@@ -14,7 +14,6 @@
 //     packed `fma.rn.f32x2` (FFMA2) on the 64-bit halves of the LDS.128 results.
 #include <cuda.h>  // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint)
 
-#include <cstdlib>
 #include <type_traits>
 
 #include "common.cuh"
@@ -301,33 +300,14 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-// (D / 4, log2 lanes per neighbour) the kernel is instantiated for: G = 4 where D/4 divides by 4, else G = 8
-#define BG_TMA_COMBOS(X) X(4, 2) X(8, 2) X(12, 2) X(16, 2) X(20, 2) X(24, 2) X(32, 2) X(10, 3) X(30, 3) X(40, 3)
-
-int launch_src_tma(const BwdParams& p, const Tiling& t, cudaStream_t st) {
-  const char* env = getenv("BOTGAT_BWD_TMA");  // read per call: the tests run every variant in one process
-  if (env && *env == '0') return 1;
-  // float4 access to ft / grad_ft (t.vw == 4), a 16-byte aligned table with rows a multiple of 16 bytes
-  if (t.vw != 4 || p.D % 8 != 0 || p.ld_g % 4 != 0 || ((uintptr_t)p.g % 16) != 0) return 1;
-  const int dv = p.D / 4;
-  const int gsh = (dv % 4 == 0 && dv <= 32) ? 2 : 3;
-  bool have = false;
-#define BG_T(DV, GSH) have = have || (dv == DV && gsh == GSH);
-  BG_TMA_COMBOS(BG_T)
-#undef BG_T
-  if (!have) return 1;
-  const bool no_eid = !p.ee && !p.amul_e && !p.keep && !p.gz_e;
-  const int mode = !no_eid ? 0 : (p.eb && p.gz && !p.am && !(p.attn_p > 0.f)) ? 1 : 2;
-  const int64_t nblocks = (int64_t)p.n_items * p.h_count;
-  if (nblocks <= 0 || nblocks >= (1ll << 31)) return 1;
-
+int launch_src_tma(const BwdParams& p, const SrcPlan& plan, cudaStream_t st) {
   static EncodeTiledFn encode = nullptr;
   if (!encode) {
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult qres;
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn) {
       cudaGetLastError();
-      return 1;
+      BG_REQUIRE(false, "backward: driver entry point cuTensorMapEncodeTiled not found");
     }
     encode = (EncodeTiledFn)fn;
   }
@@ -336,23 +316,20 @@ int launch_src_tma(const BwdParams& p, const Tiling& t, cudaStream_t st) {
   cuuint64_t gstride[1] = {(cuuint64_t)p.ld_g * 4};
   cuuint32_t box[2] = {(cuuint32_t)p.D, 1};  // tile::gather4: a box of ONE row, four row coordinates per request
   cuuint32_t estr[2] = {1, 1};
-  if (encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)p.g, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-    return 1;
-#define BG_T(DV, GSH)                                                                   \
-  if (dv == DV && gsh == GSH) {                                                         \
-    if (mode == 1)                                                                      \
-      gat_bwd_src_tma_kernel<DV, GSH, 1><<<dim3((unsigned)nblocks), dim3(32), 0, st>>>(p, tmap); \
-    else if (mode == 2)                                                                 \
-      gat_bwd_src_tma_kernel<DV, GSH, 2><<<dim3((unsigned)nblocks), dim3(32), 0, st>>>(p, tmap); \
-    else                                                                                \
-      gat_bwd_src_tma_kernel<DV, GSH, 0><<<dim3((unsigned)nblocks), dim3(32), 0, st>>>(p, tmap); \
-    BG_LAUNCHED(1);                                                                     \
-    return 0;                                                                           \
-  }
-  BG_TMA_COMBOS(BG_T)
-#undef BG_T
-  return 1;
+  const CUresult cr = encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)p.g, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  BG_REQUIRE(cr == CUDA_SUCCESS, "backward: cuTensorMapEncodeTiled failed (CUresult %d) for D=%d", (int)cr, p.D);
+  const bool launched = with_tma_combo(plan.tma_dv, plan.tma_gsh, [&](auto dv, auto gsh) {
+    if (plan.tma_mode == 1)
+      gat_bwd_src_tma_kernel<dv.value, gsh.value, 1><<<plan.grid, 32, 0, st>>>(p, tmap);
+    else if (plan.tma_mode == 2)
+      gat_bwd_src_tma_kernel<dv.value, gsh.value, 2><<<plan.grid, 32, 0, st>>>(p, tmap);
+    else
+      gat_bwd_src_tma_kernel<dv.value, gsh.value, 0><<<plan.grid, 32, 0, st>>>(p, tmap);
+  });
+  BG_REQUIRE(launched, "backward: no TMA kernel for D=%d lanes=%d", 4 * plan.tma_dv, 1 << plan.tma_gsh);
+  BG_LAUNCHED(1);
+  return 0;
 }
 
 }  // namespace botgat

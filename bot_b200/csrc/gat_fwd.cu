@@ -219,21 +219,17 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32, fwd_min_blocks(VPL)) gat_
   }
 }
 
-static int launch_fwd(const FwdParams& p, const Tiling& t, dim3 grid, cudaStream_t st) {
-  dim3 block(kWarpsPerBlock * 32);
-#define BG_X(VW, GSH, VPL)                                        \
-  if (t.vw == VW && t.gshift == GSH && t.vpl == VPL) {            \
-    if (p.ep.any())                                               \
-      gat_fwd_kernel<VW, GSH, VPL, true><<<grid, block, 0, st>>>(p);  \
-    else                                                          \
-      gat_fwd_kernel<VW, GSH, VPL, false><<<grid, block, 0, st>>>(p); \
-    BG_LAUNCHED(1);                                               \
-    return 0;                                                     \
-  }
-  BG_COMBOS(BG_X)
-#undef BG_X
-  set_error("forward: no kernel for vw=%d lanes=%d slots=%d", t.vw, 1 << t.gshift, t.vpl);
-  return -1;
+static int launch_fwd(const FwdParams& p, const FwdPlan& plan, cudaStream_t st) {
+  const Tiling& t = plan.t;
+  const bool launched = with_combo(t.vw, t.gshift, t.vpl, [&](auto vw, auto gsh, auto vpl) {
+    if (p.ep.any())
+      gat_fwd_kernel<vw.value, gsh.value, vpl.value, true><<<plan.grid, kWarpsPerBlock * 32, 0, st>>>(p);
+    else
+      gat_fwd_kernel<vw.value, gsh.value, vpl.value, false><<<plan.grid, kWarpsPerBlock * 32, 0, st>>>(p);
+  });
+  BG_REQUIRE(launched, "forward: no kernel for vw=%d lanes=%d slots=%d", t.vw, 1 << t.gshift, t.vpl);
+  BG_LAUNCHED(1);
+  return 0;
 }
 
 }  // namespace botgat
@@ -259,11 +255,6 @@ extern "C" int botgat_gat_forward(const botgat_graph* g, const botgat_fwd_args* 
   BG_REQUIRE(!a->res2 || a->ld_res2 >= HDf, "forward: ld_res2 < H*D");
   BG_REQUIRE(!a->y || a->ld_y >= HDf, "forward: ld_y < H*D");
   BG_REQUIRE(a->y || (!a->ep_scale && !a->ep_shift && !a->ep_relu), "forward: the epilogue's scale / shift / relu need y");
-  // the row-local arrays (out, residuals, y, the per-column scale / shift) constrain the vector width together
-  const int64_t ld_o = a->ld_out | (a->res ? a->ld_res : 0) | (a->res2 ? a->ld_res2 : 0) | (a->y ? a->ld_y : 0);
-  const uintptr_t p_o = (uintptr_t)a->out | (uintptr_t)a->res | (uintptr_t)a->res2 | (uintptr_t)a->y | (uintptr_t)a->ep_scale |
-                        (uintptr_t)a->ep_shift;
-  Tiling t = choose_tiling(a->H, a->D, a->ld_ft, a->ft, ld_o, (const void*)p_o, a->col_parts, g->n_src);
   FwdParams p;
   p.indptr = g->in_indptr; p.indices = g->in_indices; p.eid = g->in_eid;
   p.n_rows = (int)g->n_dst; p.n_src_table = g->n_src; p.n_edges = g->n_edges;
@@ -275,9 +266,7 @@ extern "C" int botgat_gat_forward(const botgat_graph* g, const botgat_fwd_args* 
   p.out = a->out; p.row_max = a->row_max; p.row_sum = a->row_sum;
   p.ep.res = a->res; p.ep.ld_res = a->ld_res; p.ep.res2 = a->res2; p.ep.ld_res2 = a->ld_res2;
   p.ep.scale = a->ep_scale; p.ep.shift = a->ep_shift; p.ep.relu = a->ep_relu; p.ep.y = a->y; p.ep.ld_y = a->ld_y;
-  p.col_parts = t.col_parts; p.part_cols = t.part_cols; p.omask = t.omask;
   const botgat_graph::SegTable& seg = g->seg_in;
-  const bool lowdeg = use_lowdeg_kernels(g->n_edges, g->n_dst, false);
   const bool split = seg.n_items > 0;   // both kernel families work on (row | segment) items
   BG_REQUIRE(!split || seg.n_slots == 0 || a->scratch, "forward: this graph has split rows; scratch is required");
   p.seg_row = split ? seg.row : nullptr; p.seg_beg = seg.beg; p.seg_end = seg.end; p.seg_slot = seg.slot;
@@ -287,10 +276,13 @@ extern "C" int botgat_gat_forward(const botgat_graph* g, const botgat_fwd_args* 
   p.h_count = a->h_count > 0 ? a->h_count : a->H - a->h_begin;
   BG_REQUIRE(p.h_begin >= 0 && p.h_count > 0 && p.h_begin + p.h_count <= a->H, "forward: bad head range [%d, +%d) of %d", a->h_begin, a->h_count, a->H);
   BG_REQUIRE(!split || p.h_count == a->H, "forward: a graph with split rows needs the full head range");
-  const int64_t nblocks = (int64_t)p.blocks_per_slab * p.h_count * t.col_parts;
-  BG_REQUIRE(nblocks < (1ll << 31), "forward: grid too large");
-  int rc = launch_fwd_rowwise(p, t, st);  // 1 = not wanted for this table size / shape not covered
-  if (rc == 1) rc = lowdeg ? launch_fwd_lowdeg(p, t, st) : launch_fwd(p, t, dim3((unsigned)nblocks), st);
+  FwdPlan plan;
+  int rc = plan_forward(Knobs::read(), p, a->col_parts, &plan);
+  if (rc) return rc;
+  p.col_parts = plan.t.col_parts; p.part_cols = plan.t.part_cols; p.omask = plan.t.omask;
+  rc = plan.family == Family::rowwise ? launch_fwd_rowwise(p, plan, st)
+       : plan.family == Family::lowdeg ? launch_fwd_lowdeg(p, plan, st)
+                                       : launch_fwd(p, plan, st);
   if (rc) return rc;
   if (split) {
     rc = launch_fwd_combine(seg, a->H, a->D, a->ld_out, a->scratch, a->dst_scale, a->out, a->row_max, a->row_sum, p.ep, st);

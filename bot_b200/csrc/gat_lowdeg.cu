@@ -9,23 +9,11 @@
 // gathers 32/G feature rows (one per group), so the steady-state gather rate is unchanged.
 //
 // Same math, same operand conventions and the same software pipeline as the warp-per-row kernels.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "params.cuh"
 
 namespace botgat {
 
-
-bool use_lowdeg_kernels(int64_t n_edges, int64_t n_rows, bool backward) {
-  // average neighbours per row below which a group owns a row (swept on B200, profiles/r01_sweeps.md): the
-  // forward switches late (its chunk overhead is per G neighbours instead of per 32), the backward src pass
-  // early (its per-row prologue/epilogue is heavier: ft[u] load, two outputs)
-  const char* s = getenv(backward ? "BOTGAT_LOWDEG_BWD" : "BOTGAT_LOWDEG");
-  if (!(s && *s)) s = getenv("BOTGAT_LOWDEG");
-  const int64_t thr = (s && *s) ? atoll(s) : (backward ? 96 : 20);
-  return n_rows > 0 && n_edges < thr * n_rows;
-}
 
 template <int G> __device__ __forceinline__ float group_max(float v) {
 #pragma unroll
@@ -196,26 +184,17 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32, fwd_min_blocks(VPL)) gat_
   }
 }
 
-int launch_fwd_lowdeg(const FwdParams& p, const Tiling& t, cudaStream_t st) {
-  const int rpw = 32 >> t.gshift;
-  const int warps_per_slab = (p.n_items + rpw - 1) / rpw;
-  const int64_t warps = (int64_t)warps_per_slab * p.h_count * p.col_parts;
-  const int64_t nblocks = (warps + kWarpsPerBlock - 1) / kWarpsPerBlock;
-  if (nblocks >= (1ll << 31)) { set_error("forward: grid too large"); return -1; }
-  dim3 grid((unsigned)nblocks), block(kWarpsPerBlock * 32);
-#define BG_X(VW, GSH, VPL)                                                               \
-  if (t.vw == VW && t.gshift == GSH && t.vpl == VPL) {                                   \
-    if (p.ep.any())                                                                      \
-      gat_fwd_lowdeg_kernel<VW, GSH, VPL, true><<<grid, block, 0, st>>>(p, warps_per_slab);  \
-    else                                                                                 \
-      gat_fwd_lowdeg_kernel<VW, GSH, VPL, false><<<grid, block, 0, st>>>(p, warps_per_slab); \
-    BG_LAUNCHED(1);                                                                      \
-    return 0;                                                                            \
-  }
-  BG_COMBOS(BG_X)
-#undef BG_X
-  set_error("forward: no low-degree kernel for vw=%d lanes=%d slots=%d", t.vw, 1 << t.gshift, t.vpl);
-  return -1;
+int launch_fwd_lowdeg(const FwdParams& p, const FwdPlan& plan, cudaStream_t st) {
+  const Tiling& t = plan.t;
+  const bool launched = with_combo(t.vw, t.gshift, t.vpl, [&](auto vw, auto gsh, auto vpl) {
+    if (p.ep.any())
+      gat_fwd_lowdeg_kernel<vw.value, gsh.value, vpl.value, true><<<plan.grid, kWarpsPerBlock * 32, 0, st>>>(p, plan.warps_per_slab);
+    else
+      gat_fwd_lowdeg_kernel<vw.value, gsh.value, vpl.value, false><<<plan.grid, kWarpsPerBlock * 32, 0, st>>>(p, plan.warps_per_slab);
+  });
+  BG_REQUIRE(launched, "forward: no low-degree kernel for vw=%d lanes=%d slots=%d", t.vw, 1 << t.gshift, t.vpl);
+  BG_LAUNCHED(1);
+  return 0;
 }
 
 // ---------------------------------------------------------------------------
@@ -405,23 +384,14 @@ gat_bwd_src_lowdeg_kernel(const BwdParams p, int warps_per_slab) {
   }
 }
 
-int launch_src_lowdeg(const BwdParams& p, const Tiling& t, cudaStream_t st) {
-  const int rpw = 32 >> t.gshift;
-  const int warps_per_slab = (p.n_items + rpw - 1) / rpw;
-  const int64_t warps = (int64_t)warps_per_slab * p.h_count;
-  const int64_t nblocks = (warps + kWarpsPerBlock - 1) / kWarpsPerBlock;
-  if (nblocks >= (1ll << 31)) { set_error("backward: grid too large"); return -1; }
-  dim3 grid((unsigned)nblocks), block(kWarpsPerBlock * 32);
-#define BG_X(VW, GSH, VPL)                                                                   \
-  if (t.vw == VW && t.gshift == GSH && t.vpl == VPL) {                                       \
-    gat_bwd_src_lowdeg_kernel<VW, GSH, VPL><<<grid, block, 0, st>>>(p, warps_per_slab);      \
-    BG_LAUNCHED(1);                                                                          \
-    return 0;                                                                                \
-  }
-  BG_COMBOS(BG_X)
-#undef BG_X
-  set_error("backward: no low-degree kernel for vw=%d lanes=%d slots=%d", t.vw, 1 << t.gshift, t.vpl);
-  return -1;
+int launch_src_lowdeg(const BwdParams& p, const SrcPlan& plan, cudaStream_t st) {
+  const Tiling& t = plan.t;
+  const bool launched = with_combo(t.vw, t.gshift, t.vpl, [&](auto vw, auto gsh, auto vpl) {
+    gat_bwd_src_lowdeg_kernel<vw.value, gsh.value, vpl.value><<<plan.grid, kWarpsPerBlock * 32, 0, st>>>(p, plan.warps_per_slab);
+  });
+  BG_REQUIRE(launched, "backward: no low-degree kernel for vw=%d lanes=%d slots=%d", t.vw, 1 << t.gshift, t.vpl);
+  BG_LAUNCHED(1);
+  return 0;
 }
 
 }  // namespace botgat

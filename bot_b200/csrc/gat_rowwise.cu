@@ -18,8 +18,6 @@
 // Same math, operand conventions, scratch-slot layout (split rows) and determinism as the head-major kernels.
 // Staged per-edge operands only (eb / am / gz in CSR order, in-kernel Philox); the edge-id ("direct") operand mode
 // stays on the head-major kernels.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "params.cuh"
 
@@ -493,9 +491,6 @@ __device__ __forceinline__ void rw_wait(uint32_t bar, uint32_t parity) {
       : "memory");
 }
 
-constexpr int kBulkRingLog2 = 3;  // R = 8 slots
-constexpr int kBulkRing = 1 << kBulkRingLog2;
-
 template <int GSH, int VPL>
 __global__ void __launch_bounds__(32, 10) gat_bwd_src_rowbulk_kernel(const BwdParams p, int slotB) {
   constexpr int G = 1 << GSH;
@@ -727,119 +722,43 @@ __global__ void __launch_bounds__(32, 10) gat_bwd_src_rowbulk_kernel(const BwdPa
 }
 
 // ---------------------------------------------------------------------------
-// selection and launch
+// launch
 // ---------------------------------------------------------------------------
-#define BG_RW_VPLS(X, GSH) X(GSH, 1) X(GSH, 2) X(GSH, 3) X(GSH, 4) X(GSH, 5) X(GSH, 6) X(GSH, 7) X(GSH, 8)
-#define BG_RW_COMBOS(X) BG_RW_VPLS(X, 2) BG_RW_VPLS(X, 3) BG_RW_VPLS(X, 4) BG_RW_VPLS(X, 5)
-
-// lane geometry for `heads` heads of width D: log2(lanes per head) and vector slots per lane; false = not covered
-static bool rowwise_geometry(int heads, int D, int* gsh, int* vpl) {
-  if (heads < 1 || heads > 8 || D % 4 != 0) return false;
-  int hg = 1;
-  while (hg < heads) hg <<= 1;
-  int g = 32 / hg, s = 0;
-  while ((1 << s) < g) ++s;
-  const int need = (D / 4 + g - 1) / g;
-  if (need > 8) return false;
-  *gsh = s;
-  *vpl = need;
-  return true;
+int launch_fwd_rowwise(const FwdParams& p, const FwdPlan& plan, cudaStream_t st) {
+  const bool launched = with_rw_combo(plan.rw_gsh, plan.rw_vpl, [&](auto gsh, auto vpl) {
+    if (p.ep.any())
+      gat_fwd_rowwise_kernel<gsh.value, vpl.value, true><<<plan.grid, kWarpsPerBlock * 32, 0, st>>>(p);
+    else
+      gat_fwd_rowwise_kernel<gsh.value, vpl.value, false><<<plan.grid, kWarpsPerBlock * 32, 0, st>>>(p);
+  });
+  BG_REQUIRE(launched, "forward: no row-wise kernel for lanes=%d slots=%d", 1 << plan.rw_gsh, plan.rw_vpl);
+  BG_LAUNCHED(1);
+  return 0;
 }
 
-// When the all-heads-per-row kernels are used (swept on B200 with tools/rowwise_crossover.sh, profiles/r02_sweeps.md):
-//   * never while a head's slab (one column part of it, forward) fits the L2 budget of the head-major order
-//     (BOTGAT_SLAB_MB, 64 MB): proteins / Reddit shapes stay head-major, whatever the degree;
-//   * beyond that, always for low-degree graphs (< 96 neighbours per row: 1.6 - 2x at 25 and 60 neighbours per row from a
-//     69 MB slab upwards — the head-major order pays the row's dependent load chain once per head and part);
-//   * for long rows only once the slab is well past the L2: forward from 96 MB (still 1.25x at 240 neighbours per row
-//     and a 137 MB slab), backward src pass from 256 MB (at 137 MB and >= 120 neighbours per row the TMA src pass wins).
-// BOTGAT_ROWWISE[_FWD|_BWD]=0 / 1 forces the choice (tests, sweeps); BOTGAT_ROWWISE_MB replaces both "always" sizes.
-static bool rowwise_wanted(int D, int64_t n_rows_table, int64_t n_edges, int64_t n_csr_rows, bool backward) {
-  const char* s = getenv(backward ? "BOTGAT_ROWWISE_BWD" : "BOTGAT_ROWWISE_FWD");  // read per call: the tests run every variant in one process
-  if (!(s && *s)) s = getenv("BOTGAT_ROWWISE");
-  if (s && *s) return *s != '0';
-  const char* mb = getenv("BOTGAT_ROWWISE_MB");
-  const char* sb = getenv("BOTGAT_SLAB_MB");
-  const int64_t always = ((mb && *mb) ? atoll(mb) : (backward ? 256 : 96)) << 20;
-  int64_t resident = ((sb && *sb) ? atoll(sb) : 64) << 20;
-  if (resident > always) resident = always;
-  // the forward may split a head into column parts of >= 16 vectors (choose_tiling); the src pass gathers whole heads
-  const int max_parts = (!backward && D / 64 > 0) ? D / 64 : 1;
-  const int64_t part_bytes = n_rows_table * (int64_t)D * 4 / max_parts;
-  if (part_bytes <= resident) return false;
-  // (rows of a handful of out-edges — the per-rank out-CSR of an 8-way partitioned products graph has 3 — are not what
-  // the one-warp-per-row src pass was swept on: they keep the group-per-row kernel unless the table is huge)
-  const bool low_degree = n_edges < 96 * n_csr_rows && (!backward || n_edges >= 8 * n_csr_rows);
-  return low_degree || part_bytes > always;
-}
-
-bool drec_node_major(int H, int D, int64_t n_dst, int64_t n_edges, int64_t n_src) {
-  int gsh, vpl;
-  return rowwise_wanted(D, n_dst, n_edges, n_src, true) && rowwise_geometry(H, D, &gsh, &vpl);
-}
-
-int launch_fwd_rowwise(const FwdParams& p, const Tiling& t, cudaStream_t st) {
-  int gsh, vpl;
-  if (t.vw != 4 || p.ee || p.keep || p.amul_e || !rowwise_wanted(p.D, p.n_src_table, p.n_edges, p.n_rows, false) || !rowwise_geometry(p.h_count, p.D, &gsh, &vpl))
-    return 1;
-  const int64_t nblocks = ((int64_t)p.n_items + kWarpsPerBlock - 1) / kWarpsPerBlock;
-  if (nblocks <= 0 || nblocks >= (1ll << 31)) return 1;
-#define BG_X(GSH, VPL)                                                                                       \
-  if (gsh == GSH && vpl == VPL) {                                                                            \
-    if (p.ep.any())                                                                                          \
-      gat_fwd_rowwise_kernel<GSH, VPL, true><<<dim3((unsigned)nblocks), dim3(kWarpsPerBlock * 32), 0, st>>>(p);  \
-    else                                                                                                     \
-      gat_fwd_rowwise_kernel<GSH, VPL, false><<<dim3((unsigned)nblocks), dim3(kWarpsPerBlock * 32), 0, st>>>(p); \
-    BG_LAUNCHED(1);                                                                                          \
-    return 0;                                                                                                \
-  }
-  BG_RW_COMBOS(BG_X)
-#undef BG_X
-  return 1;
-}
-
-int launch_src_rowwise(const BwdParams& p, const Tiling& t, cudaStream_t st) {
-  int gsh, vpl;
-  if (t.vw != 4 || p.ee || p.keep || p.amul_e || p.gz_e || !rowwise_wanted(p.D, p.n_dst, p.n_edges, p.n_rows, true) || !rowwise_geometry(p.h_count, p.D, &gsh, &vpl))
-    return 1;
-  const int64_t nblocks = ((int64_t)p.n_items + kWarpsPerBlock - 1) / kWarpsPerBlock;
-  if (nblocks <= 0 || nblocks >= (1ll << 31) || p.n_items <= 0) return 1;
-  // rows staged by bulk copies (one-warp blocks, shared-memory ring) unless BOTGAT_RW_BULK=0 or a staged row is too
-  // large for a ring of kBulkRing slots; the register-ring kernel otherwise
-  const char* eb = getenv("BOTGAT_RW_BULK");
-  const int slotB = (int)(((int64_t)p.h_count * p.D * 4 + 127) / 128 * 128);
-  const size_t ringB = (size_t)kBulkRing * slotB;
-  const bool bulk = !(eb && *eb == '0') && ringB <= 96 * 1024 && ((uintptr_t)p.g % 16) == 0 && p.ld_g % 4 == 0;
-  if (bulk) {
-#define BG_X(GSH, VPL)                                                                                                \
-  if (gsh == GSH && vpl == VPL) {                                                                                     \
-    static bool attr_set = false;                                                                                     \
-    if (!attr_set) {                                                                                                  \
-      if (cudaFuncSetAttribute(gat_bwd_src_rowbulk_kernel<GSH, VPL>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
-                               96 * 1024) != cudaSuccess) {                                                           \
-        cudaGetLastError();                                                                                           \
-        return 1;                                                                                                     \
-      }                                                                                                               \
-      cudaFuncSetAttribute(gat_bwd_src_rowbulk_kernel<GSH, VPL>, cudaFuncAttributePreferredSharedMemoryCarveout, 100); \
-      attr_set = true;                                                                                                \
-    }                                                                                                                 \
-    gat_bwd_src_rowbulk_kernel<GSH, VPL><<<dim3((unsigned)p.n_items), dim3(32), ringB, st>>>(p, slotB);               \
-    BG_LAUNCHED(1);                                                                                                   \
-    return 0;                                                                                                         \
-  }
-    BG_RW_COMBOS(BG_X)
-#undef BG_X
-    return 1;
-  }
-#define BG_X(GSH, VPL)                                                                                       \
-  if (gsh == GSH && vpl == VPL) {                                                                            \
-    gat_bwd_src_rowwise_kernel<GSH, VPL><<<dim3((unsigned)nblocks), dim3(kWarpsPerBlock * 32), 0, st>>>(p);  \
-    BG_LAUNCHED(1);                                                                                          \
-    return 0;                                                                                                \
-  }
-  BG_RW_COMBOS(BG_X)
-#undef BG_X
-  return 1;
+int launch_src_rowwise(const BwdParams& p, const SrcPlan& plan, cudaStream_t st) {
+  cudaError_t err = cudaSuccess;
+  const bool launched = with_rw_combo(plan.rw_gsh, plan.rw_vpl, [&](auto gsh, auto vpl) {
+    if (plan.family == Family::rowwise) {
+      gat_bwd_src_rowwise_kernel<gsh.value, vpl.value><<<plan.grid, kWarpsPerBlock * 32, 0, st>>>(p);
+      return;
+    }
+    auto* kernel = gat_bwd_src_rowbulk_kernel<gsh.value, vpl.value>;
+    static bool attr_set = false;  // one per instantiation
+    if (!attr_set) {
+      err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBulkRingMax);
+      if (err != cudaSuccess) return;
+      cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+      attr_set = true;
+    }
+    kernel<<<plan.grid, 32, plan.bulk_ring_bytes, st>>>(p, plan.bulk_slot_bytes);
+  });
+  BG_REQUIRE(launched, "backward: no row-wise kernel for lanes=%d slots=%d", 1 << plan.rw_gsh, plan.rw_vpl);
+  if (err != cudaSuccess) cudaGetLastError();  // reported here, not by the next launch
+  BG_REQUIRE(err == cudaSuccess, "backward: bulk-copy row-wise kernel: %zu bytes of shared memory refused: %s", kBulkRingMax,
+             cudaGetErrorString(err));
+  BG_LAUNCHED(1);
+  return 0;
 }
 
 }  // namespace botgat

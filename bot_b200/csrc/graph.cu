@@ -8,7 +8,6 @@
 
 #include <atomic>
 #include <cstdarg>
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -23,77 +22,6 @@ void set_error(const char* fmt, ...) {
   va_start(ap, fmt);
   vsnprintf(g_err, sizeof(g_err), fmt, ap);
   va_end(ap);
-}
-
-static int env_int(const char* name, int dflt) {
-  const char* s = getenv(name);
-  return (s && *s) ? atoi(s) : dflt;
-}
-
-static int pow2ceil(int x) {
-  int p = 1;
-  while (p < x) p <<= 1;
-  return p;
-}
-
-Tiling choose_tiling(int H, int D, int64_t ld_g, const void* pg, int64_t ld_o, const void* po, int col_parts_req,
-                     int64_t n_rows_table) {
-  constexpr int kVplCap = 8;
-  Tiling t;
-  auto ok = [&](int vw) {
-    return D % vw == 0 && ld_g % vw == 0 && ld_o % vw == 0 && ((uintptr_t)pg % (vw * 4)) == 0 &&
-           ((uintptr_t)po % (vw * 4)) == 0;
-  };
-  t.vw = ok(4) ? 4 : (ok(2) ? 2 : 1);
-  const int force_vw = env_int("BOTGAT_VW", 0);
-  if ((force_vw == 1 || force_vw == 2) && force_vw < t.vw) t.vw = force_vw;
-  const int gline = 32 / t.vw;  // lanes that cover one 128-byte line
-  // line-alignment shift is possible when every gathered row starts on a line boundary
-  bool can_align = (ld_g * 4) % 128 == 0 && ((uintptr_t)pg % 128) == 0 && env_int("BOTGAT_NOALIGN", 0) == 0;
-  // a caller that needs the head in one part (the backward src pass) gives up the shift before the shift's extra
-  // line would push the head past one pass: 32 * kVplCap vectors instead of one line fewer
-  if (col_parts_req == 1 && can_align && D > (32 * kVplCap - gline) * t.vw) can_align = false;
-  const int cap_cols = (32 * kVplCap - (can_align ? gline : 0)) * t.vw;  // widest part one warp covers in a pass
-  int parts = col_parts_req;
-  if (parts <= 0) {
-    // auto: keep one (n_rows x part_cols) slab of the gathered table within the L2 budget
-    const int64_t budget = (int64_t)env_int("BOTGAT_SLAB_MB", 64) << 20;
-    const int64_t head_bytes = n_rows_table * (int64_t)D * 4;
-    parts = (int)((head_bytes + budget - 1) / budget);
-    if (parts < 1) parts = 1;
-    const int max_parts = D / (16 * t.vw) > 0 ? D / (16 * t.vw) : 1;  // keep parts >= 16 vectors wide
-    if (parts > max_parts) parts = max_parts;
-  }
-  auto part_cols_of = [&](int np) {
-    int pc = (D + np - 1) / np;
-    return ((pc + t.vw - 1) / t.vw) * t.vw;
-  };
-  while (part_cols_of(parts) > cap_cols) ++parts;
-  t.part_cols = part_cols_of(parts);
-  t.col_parts = (D + t.part_cols - 1) / t.part_cols;
-  const int nv = (t.part_cols + t.vw - 1) / t.vw;
-  // lanes per neighbour: one 128-byte line per group and instruction (fewer when the part is narrower),
-  // more only when the part needs over kVplCap slots
-  int G = std::min(gline, pow2ceil(nv));
-  const int force_g = env_int("BOTGAT_G", 0);
-  if (force_g >= 1 && force_g <= 32 && (force_g & (force_g - 1)) == 0) G = force_g;
-  for (;; G <<= 1) {
-    t.gshift = 0;
-    while ((1 << t.gshift) < G) ++t.gshift;
-    t.omask = can_align ? std::min(G, gline) - 1 : 0;
-    // worst-case shift over all (head, part) slab starts
-    int omax = 0;
-    for (int h = 0; h < H && t.omask; ++h)
-      for (int cp = 0; cp < t.col_parts; ++cp) omax = std::max(omax, ((h * D + cp * t.part_cols) / t.vw) & t.omask);
-    const int need = (nv + omax + G - 1) / G;
-    // smallest instantiated slot count that covers the part at this group size (common.cuh BG_COMBOS)
-    t.vpl = -1;
-    for (int c = need; c <= kVplCap; ++c)
-      if (combo_supported(t.vw, t.gshift, c)) { t.vpl = c; break; }
-    if (t.vpl > 0 || G >= 32) break;
-  }
-  if (t.vpl < 0) t.vpl = kVplCap;  // unreachable: cap_cols guarantees a fit at G = 32
-  return t;
 }
 
 // ---------------------------------------------------------------------------
@@ -308,8 +236,8 @@ extern "C" int botgat_graph_create(int64_t n_src, int64_t n_dst, int64_t n_edges
   // lists (the canonical numbering) and enough neighbours per row and block.
   {
     int ts = 1, td = 1;
-    const char* force = getenv("BOTGAT_TILES");  // "ts,td" (tests / sweeps); "0" = off
-    if (force && *force) {
+    const char* force = env_str("BOTGAT_TILES");  // "ts,td" (tests / sweeps); "0" = off
+    if (force) {
       if (sscanf(force, "%d,%d", &ts, &td) != 2) ts = td = 1;
     } else if (g->in_eid_identity && n_edges >= (1 << 22) && n_src > 0 && n_dst > 0) {
       const double avg_in = (double)n_edges / n_dst, avg_out = (double)n_edges / n_src;

@@ -5,7 +5,6 @@
 // scratch slots, and a combine kernel merges them in slot order — still no atomics, still deterministic.
 #include <cub/cub.cuh>
 
-#include <cstdlib>
 
 #include "common.cuh"
 #include "params.cuh"
@@ -13,8 +12,7 @@
 namespace botgat {
 
 int segment_length() {
-  const char* s = getenv("BOTGAT_SEG");
-  const int v = (s && *s) ? atoi(s) : 2048;
+  const int v = (int)env_int("BOTGAT_SEG", 2048);
   return v < 32 ? 32 : v;
 }
 

@@ -1,10 +1,10 @@
 """Every instantiated gather kernel against the fp64 oracle, with the launch trace confirming which one ran.
 
 The layer's hot path is a set of template kernels; host code picks one instantiation per launch from the shape, the
-pointer alignment, the graph's degrees and a few knobs (``choose_tiling`` in csrc/graph.cu, ``use_lowdeg_kernels``,
-``rowwise_wanted`` / ``rowwise_geometry``, ``launch_src_tma``).  An off-by-one in the lane / slot arithmetic of one
-instantiation only shows when that instantiation runs, and a case that quietly falls back to another family still
-passes.  So each case below
+pointer alignment, the graph's degrees and a few knobs (``plan_forward`` / ``plan_src`` in csrc/plan.cu, with
+``choose_tiling``, ``rowwise_wanted`` / ``rowwise_geometry`` and the low-degree threshold).  An off-by-one in the lane /
+slot arithmetic of one instantiation only shows when that instantiation runs, and a case that quietly falls back to
+another family still passes.  So each case below
 
 * sets shape, alignment and knobs, and predicts the forward and backward src-pass instantiation with a restatement of
   the selection functions (``expected_kernels``; a drift between it and the C++ code fails the trace assertion);
@@ -41,7 +41,7 @@ KNOBS = ("BOTGAT_ROWWISE", "BOTGAT_ROWWISE_FWD", "BOTGAT_ROWWISE_BWD", "BOTGAT_R
 
 
 # ---------------------------------------------------------------------------
-# restatement of the kernel selection (csrc/common.cuh, graph.cu, gat_lowdeg.cu, gat_rowwise.cu, gat_bwd_tma.cu)
+# restatement of the kernel selection (csrc/plan.cu; the instantiation lists are in common.cuh and params.cuh)
 # ---------------------------------------------------------------------------
 def _combos():
     """BG_COMBOS (common.cuh): the head-major (VW, GSH, VPL) geometries."""
@@ -53,8 +53,8 @@ def _combos():
 
 
 COMBOS = _combos()
-TMA_COMBOS = {(4, 2), (8, 2), (12, 2), (16, 2), (20, 2), (24, 2), (32, 2), (10, 3), (30, 3), (40, 3)}  # BG_TMA_COMBOS
-BULK_RING = 8        # kBulkRing (gat_rowwise.cu)
+TMA_COMBOS = {(4, 2), (8, 2), (12, 2), (16, 2), (20, 2), (24, 2), (32, 2), (10, 3), (30, 3), (40, 3)}  # BG_TMA_COMBOS (params.cuh)
+BULK_RING = 8        # kBulkRing (params.cuh)
 
 
 def _env_int(env, name, dflt):
@@ -70,7 +70,7 @@ def _pow2ceil(x):
 
 
 def choose_tiling(H, D, ld_g, pg, ld_o, po, parts_req, n_rows, env):
-    """graph.cu choose_tiling: returns (vw, gshift, vpl, col_parts).  ``pg`` / ``po``: pointer addresses (or their
+    """plan.cu choose_tiling: returns (vw, gshift, vpl, col_parts).  ``pg`` / ``po``: pointer addresses (or their
     residues modulo 128)."""
     def ok(vw):
         return D % vw == 0 and ld_g % vw == 0 and ld_o % vw == 0 and pg % (vw * 4) == 0 and po % (vw * 4) == 0
@@ -115,12 +115,14 @@ def choose_tiling(H, D, ld_g, pg, ld_o, po, parts_req, n_rows, env):
 
 
 def use_lowdeg(n_edges, n_rows, backward, env):
+    """plan.cu low_degree with the threshold of Knobs::read."""
     s = env.get("BOTGAT_LOWDEG_BWD" if backward else "BOTGAT_LOWDEG", "") or env.get("BOTGAT_LOWDEG", "")
     thr = int(s) if s else (96 if backward else 20)
     return n_rows > 0 and n_edges < thr * n_rows
 
 
 def rowwise_geometry(heads, D):
+    """plan.cu rowwise_geometry: (log2 lanes per head, slots per lane) or None."""
     if heads < 1 or heads > 8 or D % 4:
         return None
     g = 32 // _pow2ceil(heads)
@@ -129,6 +131,7 @@ def rowwise_geometry(heads, D):
 
 
 def rowwise_wanted(D, n_rows_table, n_edges, n_csr_rows, backward, env):
+    """plan.cu rowwise_wanted."""
     s = env.get("BOTGAT_ROWWISE_BWD" if backward else "BOTGAT_ROWWISE_FWD", "") or env.get("BOTGAT_ROWWISE", "")
     if s:
         return s[0] != "0"
@@ -148,7 +151,8 @@ def _b(x):
 
 def expected_kernels(c, env, edge_mode):
     """(forward training kernel, forward inference kernel, backward src-pass kernel) for case ``c`` (see ``make_inputs``),
-    as botgat::name<args> strings."""
+    as botgat::name<args> strings: the family order of plan.cu plan_forward (row-wise, low-degree, warp) and plan_src
+    (row-wise with bulk or register ring, TMA unless low-degree, low-degree, warp)."""
     H, D, n_src, n_dst, E = c["H"], c["D"], c["n_src"], c["n_dst"], c["E"]
     direct = edge_mode == "direct"
     has_edge_ops = c["ee"] or c["keep"] or c["attn_mul"]

@@ -217,8 +217,11 @@ def test_padded_edge_records(cuda):
 @pytest.mark.parametrize("rowwise", ["0", "1"])
 @pytest.mark.parametrize("mode", ["staged", "direct"])
 def test_edge_modes_agree(cuda, monkeypatch, mode, rowwise):
-    """rowwise = 1 with the direct mode: the all-heads-per-row kernels do not take operands by edge id, so the src pass
-    falls back to the head-major kernels after the node phase already wrote node-major records (it is redone)."""
+    """Staged and direct edge operands, with and without the all-heads-per-row kernels.  Those take no operand by edge
+    id, so rowwise = 1 with the direct mode runs the head-major src pass; the plan of the src pass decides the record
+    layout before the node phase, which therefore runs exactly once per backward."""
+    from torch.profiler import ProfilerActivity, profile
+
     from bot_b200 import functional
 
     monkeypatch.setenv("BOTGAT_ROWWISE", rowwise)
@@ -226,9 +229,12 @@ def test_edge_modes_agree(cuda, monkeypatch, mode, rowwise):
     old = functional.edge_mode
     functional.edge_mode = mode
     try:
-        check_case(c, cuda)
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            check_case(c, cuda)  # one forward and one backward
+            torch.cuda.synchronize()
     finally:
         functional.edge_mode = old
+    assert sum("gat_bwd_node_kernel" in e.name for e in prof.events()) == 1
 
 
 @pytest.mark.parametrize("lowdeg", ["0", "1000000"])
@@ -1058,29 +1064,49 @@ def test_rowwise_philox(cuda, monkeypatch, H, bulk):
         assert rel_err(g[k], ref_g[k]) <= 1e-4, k
 
 
-@pytest.mark.parametrize("name", ["proteins_like_edge_drop", "products_like_H4_D120", "reddit_like_H4_D64_symm"])
+@pytest.mark.parametrize("name", ["proteins_like_edge_drop", "products_like_H4_D120", "reddit_like_H4_D64_symm",
+                                  "H12_in_halves"])
 def test_rowwise_head_range_launches(cuda, monkeypatch, name):
     """Head-range launches (the head-pipelined halo exchange's protocol) through the all-heads-per-row kernels: a range
     of heads is a narrower row; results are bit-identical to the single launch when the lane geometry is the same and
-    within rounding otherwise (fewer heads per launch -> more lanes per head -> another summation order)."""
+    within rounding otherwise (fewer heads per launch -> more lanes per head -> another summation order).
+    H12_in_halves: one launch of 12 heads is not covered by the all-heads-per-row kernels, so the node phase writes the
+    per-destination records head-major, and the two 6-head src passes run the row-wise kernel on them."""
     import bot_b200
+    from torch.profiler import ProfilerActivity, profile
+
     from bot_b200.functional import Hooks, gat_fused
+    from util import GRAD_TOL
 
     monkeypatch.setenv("BOTGAT_ROWWISE", "1")
-    n_src, n_dst, e, H, D, kw = CASES[name]
+    if name == "H12_in_halves":
+        n_src, n_dst, e, H, D, kw = 500, 500, 20000, 12, 32, dict(ee=True, keep_p=0.1)
+        chunks = [(0, 6), (6, 6)]
+    else:
+        n_src, n_dst, e, H, D, kw = CASES[name]
+        chunks = [(0, 1), (1, H - 1)]
     c = make_case(n_src, n_dst, e, H, D, seed=3, **kw)
     g = bot_b200.Graph(c["src"].to(cuda), c["dst"].to(cuda), n_src, n_dst)
     names = ["ft", "el"] + (["er"] if c.get("er") is not None else []) + (["ee"] if c.get("ee") is not None else [])
     keep = c["keep"].to(cuda) if c.get("keep") is not None else None
     cs = c["src_scale"].to(cuda) if c.get("src_scale") is not None else None
     ds = c["dst_scale"].to(cuda) if c.get("dst_scale") is not None else None
-    hooks = Hooks(head_chunks=[(0, 1), (1, H - 1)], pre_head=lambda i: None, post_src_head=lambda i, gft, gel: None)
+    hooks = Hooks(head_chunks=chunks, pre_head=lambda i: None, post_src_head=lambda i, gft, gel: None)
     res = []
     for hk in (None, hooks):
         t = {k: c[k].to(cuda).clone().requires_grad_(True) for k in names}
         am = c["attn_mul"].to(cuda) if c.get("attn_mul") is not None else None
-        out = gat_fused(g, t["ft"], t["el"], t.get("er"), t.get("ee"), keep, am, cs, ds, 0.2, 0.0, 0, hooks=hk)
-        out.backward(c["gout"].to(cuda))
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            out = gat_fused(g, t["ft"], t["el"], t.get("er"), t.get("ee"), keep, am, cs, ds, 0.2, 0.0, 0, hooks=hk)
+            out.backward(c["gout"].to(cuda))
+            torch.cuda.synchronize()
         res.append([out.detach()] + [t[k].grad for k in names])
     for a, b in zip(*res):
         assert rel_err(b, a) <= 2e-6
+    # the last (chunked) run's src passes: all heads per row, one launch per chunk
+    assert sum("gat_bwd_src_row" in e.name for e in prof.events()) == len(chunks)
+    if name == "H12_in_halves":
+        ref_out, ref_g = oracle_run(c)
+        assert rel_err(res[1][0], ref_out) <= FWD_TOL
+        for k, got in zip(names, res[1][1:]):
+            assert rel_err(got, ref_g[k]) <= GRAD_TOL, k
