@@ -10,7 +10,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("BOTGAT_LIB") or os.path.join(_HERE, "libbotgat.so")  # BOTGAT_LIB: developer A/B builds
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 c_i64p = C.POINTER(C.c_int64)
 c_vp = C.c_void_p
@@ -26,8 +26,14 @@ class GraphInfo(C.Structure):
         ("max_in_deg", C.c_int64), ("max_out_deg", C.c_int64),
         ("has_zero_in_degree", C.c_int32), ("device", C.c_int32),
         ("n_slots_in", C.c_int64), ("n_slots_out", C.c_int64),
-        ("in_eid_identity", C.c_int32), ("tiles_src", C.c_int32), ("tiles_dst", C.c_int32), ("reserved_", C.c_int32),
+        ("in_eid_identity", C.c_int32), ("tiles_src", C.c_int32), ("tiles_dst", C.c_int32),
+        ("n_seg_in", C.c_int32), ("n_seg_out", C.c_int32), ("reserved_", C.c_int32),
     ]
+
+
+class EdgeSubset(C.Structure):
+    """``botgat_edge_subset``: the kept-edge adjacency of one CSR order (device pointers)."""
+    _fields_ = [("indptr", c_vp), ("indices", c_vp), ("eid", c_vp), ("kept", c_vp), ("base", c_vp), ("seg_beg", c_vp), ("seg_end", c_vp)]
 
 
 class FwdArgs(C.Structure):
@@ -43,6 +49,7 @@ class FwdArgs(C.Structure):
         ("res", c_vp), ("ld_res", C.c_int64), ("res2", c_vp), ("ld_res2", C.c_int64),
         ("ep_scale", c_vp), ("ep_shift", c_vp), ("y", c_vp), ("ld_y", C.c_int64),
         ("ep_relu", C.c_int32), ("reserved_", C.c_int32),
+        ("subset", C.POINTER(EdgeSubset)),
     ]
 
 
@@ -58,6 +65,7 @@ class BwdArgs(C.Structure):
         ("drec", c_vp), ("gprime", c_vp), ("scratch", c_vp), ("gz", c_vp),
         ("grad_ft", c_vp), ("grad_el", c_vp), ("grad_ee", c_vp), ("ld_gee", C.c_int64), ("grad_er", c_vp),
         ("h_begin", C.c_int32), ("h_count", C.c_int32),
+        ("subset_out", C.POINTER(EdgeSubset)),
     ]
 
 
@@ -74,8 +82,9 @@ SIGNATURES = {
     "botgat_coo_to_bidirected": (C.c_int, [C.c_int64, C.c_int64, c_vp, c_vp, c_vp, c_vp, c_i64p, C.c_int, c_vp]),
     "botgat_coo_remove_self_loop": (C.c_int, [C.c_int64, c_vp, c_vp, c_vp, c_vp, c_i64p, C.c_int, c_vp]),
     "botgat_coo_add_self_loop": (C.c_int, [C.c_int64, C.c_int64, c_vp, c_vp, c_vp, c_vp, C.c_int, c_vp]),
-    "botgat_edge_stage": (C.c_int, [c_vp, C.c_int, C.c_int32, c_vp, C.c_int64, c_vp, c_vp, C.c_int64, c_vp, c_vp, c_vp]),
-    "botgat_edge_unstage": (C.c_int, [c_vp, C.c_int, C.c_int32, c_vp, c_vp, C.c_int64, c_vp]),
+    "botgat_edge_stage": (C.c_int, [c_vp, C.c_int, C.c_int32, c_vp, C.c_int64, c_vp, c_vp, C.c_int64, c_vp, c_vp,
+                                    C.POINTER(EdgeSubset), c_vp]),
+    "botgat_edge_unstage": (C.c_int, [c_vp, C.c_int, C.c_int32, c_vp, c_vp, C.c_int64, C.POINTER(EdgeSubset), c_vp]),
     "botgat_edge_reduce_dst": (C.c_int, [c_vp, C.c_int32, c_vp, C.c_int64, c_vp, c_vp, c_vp]),
     "botgat_sample_workspace_bytes": (C.c_int64, [C.c_int64]),
     "botgat_sample_count": (C.c_int, [c_vp, C.c_int64, c_vp, C.c_int32, c_vp, C.POINTER(C.c_int64), c_vp, c_vp]),

@@ -329,6 +329,9 @@ extern "C" int botgat_gat_backward(const botgat_graph* g, const botgat_bwd_args*
              "backward: grad_er needs the grad_ee buffer (it is reduced from it)");
   BG_REQUIRE(!(a->eb_out && (a->ee || a->keep)), "backward: pass edge logits either staged (eb_out) or by edge id (ee/keep)");
   BG_REQUIRE(!(a->am_out && a->attn_mul), "backward: pass the dropout multiplier either staged or by edge id");
+  // with the kept-edge subset the src pass writes gz compacted and phase 4 gives the dropped edges their zeros
+  BG_REQUIRE(!a->subset_out || (a->eb_out && (a->gz || !a->grad_ee)),
+             "backward: a kept-edge subset goes with eb_out and, for grad_ee, the gz workspace");
   const int64_t HD = (int64_t)a->H * a->D;
   BG_REQUIRE(a->ld_ft >= HD && a->ld_out >= HD && a->ld_gft >= HD, "backward: leading dimension < H*D");
   BG_REQUIRE(a->eb_out ? (a->Hb == 1 || a->Hb == a->H) : true, "backward: Hb must be 1 or H");
@@ -359,6 +362,13 @@ extern "C" int botgat_gat_backward(const botgat_graph* g, const botgat_bwd_args*
     BG_REQUIRE(!split || seg.n_slots == 0 || a->scratch, "backward: this graph has split rows; scratch is required");
     p.seg_row = split ? seg.row : nullptr; p.seg_beg = seg.beg; p.seg_end = seg.end; p.seg_slot = seg.slot;
     p.n_items = split ? seg.n_items : p.n_rows; p.scratch = a->scratch;
+    if (const botgat_edge_subset* s = a->subset_out) {
+      // the kept edges only; plan_src still sees the full graph (as the forward's plan does)
+      BG_REQUIRE(s->indptr && s->indices && (!split || (s->seg_beg && s->seg_end)), "backward: incomplete kept-edge subset");
+      BG_REQUIRE(s->eid || a->am_out || !(a->attn_p > 0.f), "backward: in-kernel attention dropout needs the subset's eid");
+      p.indptr = s->indptr; p.indices = s->indices; p.eid = s->eid;
+      if (split) { p.seg_beg = s->seg_beg; p.seg_end = s->seg_end; }
+    }
     p.blocks_per_slab = (p.n_items + kWarpsPerBlock - 1) / kWarpsPerBlock;
     p.h_begin = a->h_begin;
     p.h_count = a->h_count > 0 ? a->h_count : a->H - a->h_begin;
@@ -393,7 +403,7 @@ extern "C" int botgat_gat_backward(const botgat_graph* g, const botgat_bwd_args*
   }
 
   if ((phases & 4) && a->grad_ee && a->gz && g->n_edges > 0) {
-    int rc = botgat_edge_unstage(g, BOTGAT_ORDER_OUT, a->H, a->gz, a->grad_ee, ld_gee, stream);
+    int rc = botgat_edge_unstage(g, BOTGAT_ORDER_OUT, a->H, a->gz, a->grad_ee, ld_gee, a->subset_out, stream);
     if (rc) return rc;
   }
   if ((phases & 4) && a->grad_er) {

@@ -271,6 +271,15 @@ extern "C" int botgat_gat_forward(const botgat_graph* g, const botgat_fwd_args* 
   BG_REQUIRE(!split || seg.n_slots == 0 || a->scratch, "forward: this graph has split rows; scratch is required");
   p.seg_row = split ? seg.row : nullptr; p.seg_beg = seg.beg; p.seg_end = seg.end; p.seg_slot = seg.slot;
   p.n_items = split ? seg.n_items : p.n_rows; p.scratch = a->scratch;
+  if (const botgat_edge_subset* s = a->subset) {
+    // the kept edges only; the plan below still sees the full graph (n_edges, n_rows, the table), so every call picks the
+    // kernel it picks without the subset
+    BG_REQUIRE(a->eb, "forward: a kept-edge subset goes with the edge logits staged with it (eb)");
+    BG_REQUIRE(s->indptr && s->indices && (!split || (s->seg_beg && s->seg_end)), "forward: incomplete kept-edge subset");
+    BG_REQUIRE(s->eid || a->am || !(a->attn_p > 0.f), "forward: in-kernel attention dropout needs the subset's eid");
+    p.indptr = s->indptr; p.indices = s->indices; p.eid = s->eid;
+    if (split) { p.seg_beg = s->seg_beg; p.seg_end = s->seg_end; }
+  }
   p.blocks_per_slab = (p.n_items + kWarpsPerBlock - 1) / kWarpsPerBlock;
   p.h_begin = a->h_begin;
   p.h_count = a->h_count > 0 ? a->h_count : a->H - a->h_begin;

@@ -301,7 +301,8 @@ extern "C" int botgat_graph_get_info(const botgat_graph* g, botgat_graph_info* i
   info->max_in_deg = g->max_in_deg; info->max_out_deg = g->max_out_deg;
   info->has_zero_in_degree = g->has_zero_in_degree; info->device = g->device;
   info->n_slots_in = g->seg_in.n_slots; info->n_slots_out = g->seg_out.n_slots;
-  info->in_eid_identity = g->in_eid_identity; info->tiles_src = g->tiles_s; info->tiles_dst = g->tiles_d; info->reserved_ = 0;
+  info->in_eid_identity = g->in_eid_identity; info->tiles_src = g->tiles_s; info->tiles_dst = g->tiles_d;
+  info->n_seg_in = g->seg_in.n_items; info->n_seg_out = g->seg_out.n_items; info->reserved_ = 0;
   return 0;
 }
 

@@ -61,20 +61,6 @@ timer = None  # set to a KernelTimer to record
 #             in the staging pass); kept for graphs whose edge ids already follow the CSR order.
 edge_mode = "staged"
 
-# Optionally stage the backward's (out-CSR-ordered) edge operands already during the forward, on a side stream (the
-# staging pass is DRAM-bound, the forward gather L2-bound).  Measured NEUTRAL on B200 (18.79 ms/step either way: the
-# forward kernel fills every SM, the side-stream blocks only trickle in) and it keeps one (Hb, E) buffer alive
-# until backward, so it is off by default.
-prestage_backward = False
-_side_streams = {}
-
-
-def _side_stream(device):
-    key = (device.type, device.index)
-    if key not in _side_streams:
-        _side_streams[key] = torch.cuda.Stream(device=device)
-    return _side_streams[key]
-
 
 def _span(name):
     return _Span(timer, name)
@@ -116,9 +102,38 @@ def pad_heads(H):
     return w if H <= 8 else (H + 3) // 4 * 4
 
 
-def edge_stage(graph: Graph, order, H, ee=None, keep=None, attn_mul=None):
+class KeptEdges:
+    """The CSR of one step's kept edges in one order (``botgat_edge_subset``), filled by :func:`edge_stage`.  The gather
+    kernels walk it instead of the graph's CSR, so that an edge dropped this step costs them no traffic.  Arrays keep
+    their full-graph sizes (the kept count stays on the device); ``eid`` only when a kernel reads edge ids."""
+
+    def __init__(self, graph, order, with_eid):
+        graph._ensure()
+        info, dev, E = graph._info, graph.device, graph.number_of_edges()
+        inn = order == _lib.ORDER_IN
+        rows = graph.number_of_dst_nodes() if inn else graph.number_of_src_nodes()
+        n_seg = info.n_seg_in if inn else info.n_seg_out
+
+        def i32(n):
+            return torch.empty(n, dtype=torch.int32, device=dev)
+
+        W = E // 32 + 1   # kept-flag words (botgat_edge_subset.kept / base)
+        self.kept = torch.empty(W, dtype=torch.int32, device=dev)   # uint32 bits, held as int32
+        self.base, self.indptr, self.indices = i32(W), i32(rows + 1), i32(E)
+        self.eid = i32(E) if with_eid else None
+        self.seg_beg, self.seg_end = (i32(n_seg), i32(n_seg)) if n_seg else (None, None)
+        self.c = _lib.EdgeSubset(*(None if t is None else t.data_ptr() for t in (
+            self.indptr, self.indices, self.eid, self.kept, self.base, self.seg_beg, self.seg_end)))
+
+    def ptr(self):
+        return C.pointer(self.c)
+
+
+def edge_stage(graph: Graph, order, H, ee=None, keep=None, attn_mul=None, kept=False, kept_eid=False):
     """Permute per-edge operands from edge-id order to CSR order, head-major
-    (``botgat_edge_stage``).  ``ee`` / ``attn_mul`` may be (E, >=H) with padded rows.  Returns (eb, Hb, am)."""
+    (``botgat_edge_stage``).  ``ee`` / ``attn_mul`` may be (E, >=H) with padded rows.  With ``kept`` and a ``keep`` mask,
+    also builds the adjacency of the kept edges (:class:`KeptEdges`, with edge ids when ``kept_eid``) and stages eb / am
+    compacted to it.  Returns (eb, Hb, am, KeptEdges | None)."""
     E = graph.number_of_edges()
     dev = graph.device
     eb = am = None
@@ -129,14 +144,16 @@ def edge_stage(graph: Graph, order, H, ee=None, keep=None, attn_mul=None):
     if attn_mul is not None:
         am = torch.empty((H, E), dtype=torch.float32, device=dev)
     if eb is None and am is None:
-        return None, 0, None
+        return None, 0, None, None
+    sub = KeptEdges(graph, order, kept_eid) if kept and keep is not None else None
     ee, ld_ee = _rows(ee, "ee", H)
     attn_mul, ld_am = _rows(attn_mul, "attn_mul", H)
     with _span("edge_stage"):
         rc = _lib.load().botgat_edge_stage(graph._ensure(), order, H, _lib.ptr(ee), ld_ee, _lib.ptr(keep),
-                                           _lib.ptr(attn_mul), ld_am, _lib.ptr(eb), _lib.ptr(am), _stream())
+                                           _lib.ptr(attn_mul), ld_am, _lib.ptr(eb), _lib.ptr(am),
+                                           sub.ptr() if sub is not None else None, _stream())
     _lib.check(rc, "botgat_edge_stage")
-    return eb, Hb, am
+    return eb, Hb, am, sub
 
 
 def _check_edge_operands(graph, H, ee, keep, attn_mul):
@@ -156,7 +173,8 @@ def _forward_core(graph, ft2d, H, D, el, er, ee, ld_ee, keep, attn_mul, ld_am, s
                   hooks, will_backward, ep=None):
     """Edge staging + the fused forward kernel.  ``ft2d``: 2-D tensor whose first H*D columns are the projected source
     features (any 16-byte-aligned row stride: a column slice of a wider GEMM output works).  Returns
-    (out (N_d,H,D), row_max, row_sum, prestaged backward operands | None, attn_p actually used).
+    (out (N_d,H,D), row_max, row_sum, attn_p actually used).  With a ``keep`` mask the kernels walk the kept edges only
+    (:class:`KeptEdges`).
     ``ep``: fused layer epilogue of an inference forward (``botgat_fwd_args.res`` ...): a dict with optional 2-D
     ``res`` / ``res2`` (N_d, >= H*D), ``scale`` / ``shift`` (H*D), ``relu``, ``want_y``; the ``y`` tensor is stored
     back into it."""
@@ -165,21 +183,9 @@ def _forward_core(graph, ft2d, H, D, el, er, ee, ld_ee, keep, attn_mul, ld_am, s
     dev = ft2d.device
     N_d = graph.number_of_dst_nodes()
     staged = edge_mode == "staged"
-    eb_in, Hb, am_in = edge_stage(graph, _lib.ORDER_IN, H, ee, keep, attn_mul) if staged else (None, 0, None)
-    pre = None
-    has_edge_ops = ee is not None or keep is not None or attn_mul is not None
-    if staged and prestage_backward and has_edge_ops and will_backward:
-        # after the in-order staging (both are DRAM-bound), so that it runs beside the forward gather
-        main, side = torch.cuda.current_stream(), _side_stream(dev)
-        side.wait_stream(main)
-        with torch.cuda.stream(side):
-            eb_o, _, am_o = edge_stage(graph, _lib.ORDER_OUT, H, ee, keep, attn_mul)
-            ev = torch.cuda.Event()
-            ev.record(side)
-        for t in (ee, keep, attn_mul):
-            if t is not None:
-                t.record_stream(side)
-        pre = (eb_o, am_o, ev)
+    philox = attn_mul is None and attn_p > 0   # the in-kernel dropout reads edge ids
+    eb_in, Hb, am_in, kept = (edge_stage(graph, _lib.ORDER_IN, H, ee, keep, attn_mul, kept=True, kept_eid=philox)
+                              if staged else (None, 0, None, None))
     out = torch.empty((N_d, H, D), dtype=torch.float32, device=dev)
     row_max = torch.empty((N_d, H), dtype=torch.float32, device=dev)
     row_sum = torch.empty((N_d, H), dtype=torch.float32, device=dev)
@@ -188,6 +194,8 @@ def _forward_core(graph, ft2d, H, D, el, er, ee, ld_ee, keep, attn_mul, ld_am, s
     a.ft, a.el, a.er = ft2d.data_ptr(), el.data_ptr(), (er.data_ptr() if er is not None else None)
     a.eb, a.Hb, a.col_parts = (eb_in.data_ptr() if eb_in is not None else None), Hb, 0
     a.am = am_in.data_ptr() if am_in is not None else None
+    if kept is not None:
+        a.subset = kept.ptr()
     if not staged:
         if (ee is not None and ld_ee != H) or (attn_mul is not None and ld_am != H):
             raise ValueError("direct edge mode needs unpadded (E,H) edge operands")
@@ -234,10 +242,10 @@ def _forward_core(graph, ft2d, H, D, el, er, ee, ld_ee, keep, attn_mul, ld_am, s
         with _span("gat_fwd"):
             rc = lib.botgat_gat_forward(h, C.byref(a), _stream())
         _lib.check(rc, "botgat_gat_forward")
-    return out, row_max, row_sum, pre, float(a.attn_p)
+    return out, row_max, row_sum, float(a.attn_p)
 
 
-def _backward_core(graph, cfg, pre, hooks, ft2d, el, er, ee, keep, attn_mul, src_scale, dst_scale, out, row_max, row_sum,
+def _backward_core(graph, cfg, hooks, ft2d, el, er, ee, keep, attn_mul, src_scale, dst_scale, out, row_max, row_sum,
                    gout, grad_ft2d, need_er, need_ee, hook_grad_ft=None):
     """The three backward phases.  ``grad_ft2d``: 2-D tensor whose first H*D columns receive grad_ft (any aligned row
     stride).  Returns (grad_el (N_s,H), grad_er | None, grad_ee | None)."""
@@ -250,16 +258,9 @@ def _backward_core(graph, cfg, pre, hooks, ft2d, el, er, ee, keep, attn_mul, src
     def p(t):
         return t.data_ptr() if t is not None else None
 
-    if pre is not None:  # staged during the forward on the side stream
-        eb_out, am_out, ev = pre
-        cur = torch.cuda.current_stream()
-        cur.wait_event(ev)
-        for t in (eb_out, am_out):
-            if t is not None:
-                t.record_stream(cur)
-        Hb = eb_out.shape[0] if eb_out is not None else 0
-    else:
-        eb_out, Hb, am_out = edge_stage(graph, _lib.ORDER_OUT, H, ee, keep, attn_mul) if staged else (None, 0, None)
+    philox = attn_mul is None and attn_p > 0
+    eb_out, Hb, am_out, kept = (edge_stage(graph, _lib.ORDER_OUT, H, ee, keep, attn_mul, kept=True, kept_eid=philox)
+                                if staged else (None, 0, None, None))
     drec = torch.empty((H, N_d, 4), dtype=torch.float32, device=dev)
     gprime = torch.empty_like(gout) if dst_scale is not None else None
     grad_el = torch.empty((N_s, H), dtype=torch.float32, device=dev)
@@ -281,6 +282,8 @@ def _backward_core(graph, cfg, pre, hooks, ft2d, el, er, ee, keep, attn_mul, src
     a.slope, a.attn_p, a.seed = slope, attn_p, seed
     a.out, a.row_max, a.row_sum, a.gout = out.data_ptr(), row_max.data_ptr(), row_sum.data_ptr(), gout.data_ptr()
     a.drec, a.gprime, a.gz = drec.data_ptr(), p(gprime), p(gz)
+    if kept is not None:
+        a.subset_out = kept.ptr()
     scratch = None
     if graph._info.n_slots_out or graph._info.n_slots_in:
         scratch = torch.empty(graph._info.n_slots_out * _r4(H * (D + 1)) + graph._info.n_slots_in * H,
@@ -373,12 +376,11 @@ class GATFusedFn(torch.autograd.Function):
                 Dk = _r4(D)
                 ft = torch.cat([ft, ft.new_zeros(N_s, H, Dk - D)], 2)
         with torch.cuda.device(ft.device):
-            out, row_max, row_sum, pre, attn_p_used = _forward_core(
+            out, row_max, row_sum, attn_p_used = _forward_core(
                 graph, ft.view(N_s, H * Dk), H, Dk, el, er, ee, ld_ee, keep, attn_mul, ld_am, src_scale, dst_scale, slope,
                 attn_p, seed, hooks, any(ctx.needs_input_grad))
         ctx.graph = graph
         ctx.hooks = hooks
-        ctx.pre = pre
         ctx.D = D
         ctx.cfg = (H, Dk, edge_mode == "staged", float(slope), attn_p_used, int(seed))
         ctx.save_for_backward(ft, el, er, ee, keep, attn_mul, src_scale, dst_scale, out, row_max, row_sum)
@@ -398,7 +400,7 @@ class GATFusedFn(torch.autograd.Function):
         grad_ft = torch.empty_like(ft)
         with torch.cuda.device(ft.device):
             grad_el, grad_er, grad_ee = _backward_core(
-                ctx.graph, ctx.cfg, ctx.pre, ctx.hooks, ft.view(-1, H * D), el, er, ee, keep, attn_mul, src_scale, dst_scale,
+                ctx.graph, ctx.cfg, ctx.hooks, ft.view(-1, H * D), el, er, ee, keep, attn_mul, src_scale, dst_scale,
                 out, row_max, row_sum, gout, grad_ft.view(-1, H * D), need_er, need_ee, hook_grad_ft=grad_ft)
         if D != ctx.D:
             grad_ft = grad_ft[:, :, :ctx.D]
@@ -453,11 +455,11 @@ class GATConvSampledFn(torch.autograd.Function):
             Yd = torch.addmm(bd, x_dst, wd.t())
             el = Ys[:, HD:HD + H].contiguous() if src_scale is None else Ys[:, HD:HD + H] * src_scale.unsqueeze(-1)
             er = Yd[:, HD:HD + H].contiguous() if has_er else None
-            out, row_max, row_sum, pre, attn_p_used = _forward_core(
+            out, row_max, row_sum, attn_p_used = _forward_core(
                 graph, Ys, H, D, el, er, ee, ld_ee, keep, attn_mul, ld_am, src_scale, dst_scale, slope, attn_p, seed, None,
                 any(ctx.needs_input_grad))
             rst = out + Yd[:, :HD].view(N_d, H, D)                                    # models.py:159-160
-        ctx.graph, ctx.pre, ctx.same_x = graph, pre, x_dst is x_src or x_dst.data_ptr() == x_src.data_ptr() and N_s == N_d
+        ctx.graph, ctx.same_x = graph, x_dst is x_src or x_dst.data_ptr() == x_src.data_ptr() and N_s == N_d
         ctx.cfg = (H, D, edge_mode == "staged", float(slope), attn_p_used, int(seed))
         ctx.dims = (P, has_er, w_src.shape[0], w_dst.shape[0])
         ctx.save_for_backward(x_src, x_dst, ws, wd, Ys, el, er, ee, keep, attn_mul, dst_scale, out, row_max, row_sum, src_scale)
@@ -478,7 +480,7 @@ class GATConvSampledFn(torch.autograd.Function):
             gYs = torch.empty((N_s, P), dtype=torch.float32, device=dev)
             gYd = torch.empty((N_d, P), dtype=torch.float32, device=dev)
             grad_el, grad_er, grad_ee = _backward_core(
-                ctx.graph, ctx.cfg, ctx.pre, None, Ys, el, er, ee, keep, attn_mul, src_scale, dst_scale, out, row_max, row_sum,
+                ctx.graph, ctx.cfg, None, Ys, el, er, ee, keep, attn_mul, src_scale, dst_scale, out, row_max, row_sum,
                 grst, gYs, has_er, need_ee)
             gYs[:, HD:HD + H] = grad_el if src_scale is None else grad_el * src_scale.unsqueeze(-1)
             gYs[:, HD + H:].zero_()
@@ -555,7 +557,7 @@ def gat_fused_inference(graph, ft, el, er, ee, keep, attn_mul, src_scale, dst_sc
             res = _f32c(res, "res").view(res.shape[0], -1)
         ep = {"res": res, "res2": h_last, "scale": scale, "shift": shift, "relu": tail.relu, "want_y": True}
         with torch.cuda.device(ft.device):
-            out, _, _, _, _ = _forward_core(graph, ft.view(N_s, H * D), H, D, el, er, ee, ld_ee, keep, attn_mul, ld_am, src_scale,
+            out, _, _, _ = _forward_core(graph, ft.view(N_s, H * D), H, D, el, er, ee, ld_ee, keep, attn_mul, ld_am, src_scale,
                                             dst_scale, slope, 0.0, 0, None, False, ep=ep)
         return out.view(N_d, H * D), ep["y"]
 
@@ -587,7 +589,7 @@ def gat_conv_inference(graph, x_src, x_dst, w_src, w_dst, b_dst, ee, keep, attn_
             ep["res"] = Yd                                                    # models.py:159-160, read in place
             el = Ys[:, HD:HD + H].contiguous() if src_scale is None else Ys[:, HD:HD + H] * src_scale.unsqueeze(-1)
             er = Yd[:, HD:HD + H].contiguous() if has_er else None
-            out, _, _, _, _ = _forward_core(graph, Ys, H, D, el, er, ee, ld_ee, keep, attn_mul, ld_am, src_scale, dst_scale,
+            out, _, _, _ = _forward_core(graph, Ys, H, D, el, er, ee, ld_ee, keep, attn_mul, ld_am, src_scale, dst_scale,
                                             slope, 0.0, 0, None, False, ep=ep)
         return out.view(N_d, HD), ep["y"]
 

@@ -258,7 +258,7 @@ class _P2PGatFn(torch.autograd.Function):
 
         ee, ld_ee, keep, attn_mul, ld_am = Fn._check_edge_operands(graph, H, ee, keep, attn_mul)
         hooks = Fn.Hooks(pre_kernel=pre_kernel, head_chunks=chunks, pre_head=pre_head)
-        out, row_max, row_sum, pre, attn_p_used = Fn._forward_core(
+        out, row_max, row_sum, attn_p_used = Fn._forward_core(
             graph, hx.table, H, D, el_all, er, ee, ld_ee, keep, attn_mul, ld_am, src_scale, dst_scale, slope, attn_p, seed,
             hooks, True)
         ctx.pg, ctx.hx, ctx.chunks = pg, hx, chunks
@@ -303,7 +303,7 @@ class _P2PGatFn(torch.autograd.Function):
         need_er = er is not None and ctx.needs_input_grad[5]
         need_ee = ee is not None and ctx.needs_input_grad[6]
         grad_el, grad_er, grad_ee = Fn._backward_core(
-            pg.local, ctx.cfg, None, hooks, hx.table, el_all, er, ee, keep, attn_mul, src_scale, dst_scale, out, row_max, row_sum,
+            pg.local, ctx.cfg, hooks, hx.table, el_all, er, ee, keep, attn_mul, src_scale, dst_scale, out, row_max, row_sum,
             gout, hx.gtable, need_er, need_ee)
         main.wait_stream(hx.stream)
         grad_ft_own = gshard[:n_own, :HD].unflatten(1, (H, D))

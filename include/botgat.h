@@ -31,7 +31,7 @@ extern "C" {
 #pragma GCC visibility push(default) /* the library is built with -fvisibility=hidden */
 #endif
 
-#define BOTGAT_ABI_VERSION 4
+#define BOTGAT_ABI_VERSION 5
 
 typedef struct botgat_graph botgat_graph;
 
@@ -97,6 +97,9 @@ typedef struct {
   /* cache-blocked out-CSR traversal used by botgat_edge_stage / botgat_edge_unstage(BOTGAT_ORDER_OUT):
    * tiles_src x tiles_dst node blocks (1 x 1 = plain order) */
   int32_t tiles_src, tiles_dst;
+  /* row segments (work items) of the in- / out-CSR when it has split rows, else 0: the length of
+   * botgat_edge_subset.seg_beg / seg_end (ABI v5) */
+  int32_t n_seg_in, n_seg_out;
   int32_t reserved_;
 } botgat_graph_info;
 int botgat_graph_get_info(const botgat_graph* g, botgat_graph_info* info /* HOST */);
@@ -139,13 +142,41 @@ enum { BOTGAT_ORDER_IN = 0, BOTGAT_ORDER_OUT = 1 };
  * A row stride of 8 floats (32 bytes) makes every H<=8 record one aligned DRAM sector; the kernels use the
  * widest vector access the stride and alignment allow.
  */
+/*
+ * Per-step kept adjacency (ABI v5).  Edge drop removes a tenth or more of the edges every step; the gather kernels
+ * walk this CSR of the kept edges instead of the graph's, so that a dropped edge costs them nothing.  All arrays are
+ * caller-owned and keep their full-graph sizes; E' (the kept count) stays on the device.  For the CSR named by
+ * `order` (rows = n_dst for BOTGAT_ORDER_IN, n_src for BOTGAT_ORDER_OUT), with W = n_edges/32 + 1 words and
+ * rank(x) = base[x/32] + popcount(kept[x/32] & ((1 << x%32) - 1)), the kept positions before x:
+ *   kept     (W) uint32   kept flags in CSR position order: bit p%32 of word p/32 (positions >= n_edges: 0)
+ *   base     (W) int32    kept positions before word w (exclusive scan of the words' popcounts)
+ *                         a kept position p moves to rank(p)
+ *   indptr   (rows+1)     indptr[r] = rank(graph indptr[r])
+ *   indices  (n_edges)    the kept entries in CSR order (first E' written)
+ *   eid      (n_edges)    their edge ids, or NULL; needed when a kernel reads edge ids (in-kernel attention dropout)
+ *   seg_beg, seg_end      (n_seg_in / n_seg_out of botgat_graph_info) the row segments translated through rank, or
+ *                         NULL when the CSR has no split rows
+ */
+typedef struct {
+  int32_t* indptr;
+  int32_t* indices;
+  int32_t* eid;
+  uint32_t* kept;
+  int32_t* base;
+  int32_t* seg_beg;
+  int32_t* seg_end;
+} botgat_edge_subset;
+/* With `subset` (requires keep): also fills the kept adjacency, and eb / am are written compacted, eb[hb][rank(p)] for
+ * the kept positions only (no -inf markers; the rows keep their stride n_edges).  NULL: the layout above. */
 int botgat_edge_stage(const botgat_graph* g, int order, int32_t H,
                       const float* ee, int64_t ld_ee, const uint8_t* keep,
                       const float* attn_mul, int64_t ld_am,
-                      float* eb, float* am, void* stream);
-/* grad_ee[eid(p)*ld_gee + h] = gz[h][p]  (gz head-major in the CSR order named by `order`) */
+                      float* eb, float* am, botgat_edge_subset* subset /* HOST struct or NULL */, void* stream);
+/* grad_ee[eid(p)*ld_gee + h] = gz[h][p]  (gz head-major in the CSR order named by `order`).  With `subset` (the one
+ * botgat_edge_stage filled), gz is compacted: kept p reads gz[h][rank(p)], a dropped edge gets zeros. */
 int botgat_edge_unstage(const botgat_graph* g, int order, int32_t H, const float* gz,
-                        float* grad_ee, int64_t ld_gee, void* stream);
+                        float* grad_ee, int64_t ld_gee, const botgat_edge_subset* subset /* HOST or NULL */,
+                        void* stream);
 /* grad_er[v,h] = sum over the in-edges k of v of grad_ee[k*ld_gee + h]   (replaces the copy_e/sum SpMM DGL
  * runs as the backward of u_add_v, SURVEY.md Appendix B) */
 int botgat_edge_reduce_dst(const botgat_graph* g, int32_t H, const float* grad_ee, int64_t ld_gee,
@@ -253,6 +284,9 @@ typedef struct {
   int64_t ld_y;
   int32_t ep_relu;        /* 1: y = max(., 0); needs y */
   int32_t reserved_;
+  /* kept in-CSR adjacency from botgat_edge_stage(BOTGAT_ORDER_IN, subset), or NULL = the graph's (ABI v5); eb / am
+   * must then be the compacted ones staged with it */
+  const botgat_edge_subset* subset;
 } botgat_fwd_args;
 int botgat_gat_forward(const botgat_graph* g, const botgat_fwd_args* a /* HOST */, void* stream);
 
@@ -304,6 +338,9 @@ typedef struct {
   float* grad_er;         /* (n_dst, H) or NULL */
   /* head range of the src phase (phases & 2), as in botgat_fwd_args; the node and edge phases always cover all heads */
   int32_t h_begin, h_count;
+  /* kept out-CSR adjacency from botgat_edge_stage(BOTGAT_ORDER_OUT, subset), or NULL = the graph's (ABI v5); eb_out /
+   * am_out must be the compacted ones staged with it, gz is written compacted and phase 4 un-stages it through it */
+  const botgat_edge_subset* subset_out;
 } botgat_bwd_args;
 int botgat_gat_backward(const botgat_graph* g, const botgat_bwd_args* a /* HOST */, void* stream);
 
